@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — env-steps/s of the RoboRugby step()/reset() hot path on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--preset GAME|TRAIN]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--preset GAME|TRAIN] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (BASELINE.json configs[2]): RoboRugbySimpleDuel-v2, 65 536 envs per GPU, shipped (GAME)
@@ -34,6 +34,9 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+# the tree may be read-only: no bytecode caches there, from this process or the oracle's timing subprocess
+sys.dont_write_bytecode = True
+os.environ["PYTHONDONTWRITEBYTECODE"] = "1"
 
 ENV_ID = "RoboRugbySimpleDuel-v2"
 ENVS_PER_GPU = 65536
@@ -63,6 +66,10 @@ PY_REFERENCE_NOTE = {"GAME": "Python reference (oracle/time_reference.py, build 
                      "TRAIN": "Python reference (oracle/time_reference.py, build container, 8 cores): 4467 env-steps/s (657 per core)"}
 METRIC = "env_steps_per_sec"
 UNIT = "env-steps/s"
+# --dump-outputs: the rows of a fixed sample of envs (np.random.default_rng(0), sorted), so that two builds can be compared
+# output for output without writing the whole batch (65 536 envs x 32 steps of four outputs is ~110 MB)
+DUMP_ENVS = 8192
+DUMP_BYTES = 64_000_000
 
 
 def _peaks():
@@ -174,6 +181,22 @@ def run_dqn(args, rank, world, local_rank):
                                              "step, batch 2500 (BASELINE configs[4])"}, "dqn": r}), flush=True)
 
 
+def dump_outputs(path, outs, n_envs):
+    """Write the outputs of one step_k call (obs_h, obs_g [K, N, D], rew [K, N, 2], done [K, N]) as float32 .npy files,
+    restricted to the sampled envs."""
+    import numpy as np
+    import torch
+    names = ("obs_h", "obs_g", "rew", "done")
+    per_env = 4 * sum(x[:, :1].numel() for x in outs)
+    n = max(1, min(n_envs, DUMP_ENVS, DUMP_BYTES // per_env))
+    idx = np.sort(np.random.default_rng(0).choice(n_envs, n, replace=False))
+    sel = torch.as_tensor(idx, device=outs[0].device)
+    os.makedirs(path, exist_ok=True)
+    for name, x in zip(names, outs):
+        if x.numel():   # (no observation arrays for an observer-less env id)
+            np.save(os.path.join(path, name + ".npy"), x[:, sel].float().cpu().numpy())
+
+
 def workload_config(args, world):
     return {"workload": f"{args.env_id} {args.preset} preset, {args.envs} envs/GPU x {world} GPU, random "
                         f"{'continuous thrust' if args.env_id == 'RoboRugby-v0' else 'discrete'} actions, "
@@ -205,7 +228,11 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="skip the K = 1 and DQN-loop extras")
     ap.add_argument("--workload", default="rollout", choices=["rollout", "dqn"], help="dqn: BASELINE configs[4], the "
                     "Training_DQN_pytorch loop on the GPU VecEnv (TRAIN constants, as the reference script requires)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed calls, write what the last one returned "
+                    "(obs_h, obs_g, rew, done of a fixed sample of rank 0's envs, float32) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -289,11 +316,13 @@ def main():
     t_wall0 = time.perf_counter()
     e0.record()
     for s in range(args.steps):
-        env.step_k(acts[s % n_sets], K, join=False)
+        outs = env.step_k(acts[s % n_sets], K, join=False)
     env.join()
     e1.record()
     barrier()
     t_wall = time.perf_counter() - t_wall0
+    if args.dump_outputs and rank == 0:   # before the calls below reuse the output buffers
+        dump_outputs(args.dump_outputs, outs, n_local)
     launches = env.launch_count - launches0
     my_ms = e0.elapsed_time(e1)
     kernel_ms = [my_ms / args.steps] * args.steps

@@ -13,8 +13,8 @@ from roborugby_b200._lib import Config, ABI_VERSION
 _HERE = os.path.dirname(os.path.abspath(__file__))
 _ROOT = os.path.dirname(os.path.dirname(_HERE))
 _LIB = os.path.join(_HERE, "librr_emul.so")
-_SRCS = [os.path.join(_HERE, "rr_emul.cu"), os.path.join(_ROOT, "roborugby_b200", "csrc", "rr_sim.cuh"),
-         os.path.join(_ROOT, "include", "rr_b200.h")]
+_SRCS = [os.path.join(_HERE, "rr_emul.cu"), os.path.join(_ROOT, "include", "rr_b200.h")] + [
+    os.path.join(_ROOT, "roborugby_b200", "csrc", f) for f in ("rr_sim.cuh", "rr_sincos.cuh", "rr_sincos_grid.inc")]
 
 
 def build(force=False):
