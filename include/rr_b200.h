@@ -78,7 +78,10 @@ extern "C" {
 #define RR_ERR_COINCIDENT_BALLS 64u /* RR_TrashyPhysics.py:249-250 */
 #define RR_ERR_DIV0 128u            /* MyUtils.py:25         */
 #define RR_ERR_RESET_PLACEMENT 256u /* placement loop exceeded its bound (reference: unbounded) */
-#define RR_ERR_BAD_ACTION 512u      /* discrete action id > 7: KeyError in thrust_from_direction before anything moves, RR_EnvBase.py:593-606, :624 */
+#define RR_ERR_BAD_ACTION 512u      /* an action the env cannot apply, refused before anything moves: a discrete id > 7
+                                       (KeyError in thrust_from_direction, RR_EnvBase.py:593-606, :624), or a thrust whose
+                                       int(round(x)) is NaN or +-inf (round() raises, RR_Robot.py:100-102) or lies outside
+                                       [-8, 7] (the reference would simulate it; the action space is Box(-1, 1)) */
 
 /* return codes */
 #define RR_OK 0
@@ -156,7 +159,7 @@ int rr_reset_fixed(rr_sim *s, const uint8_t *mask_dev, int32_t as_constructed, v
 int rr_set_starting_positions(rr_sim *s, const double *rob3, const double *ball2);
 int rr_get_starting_positions(rr_sim *s, double *rob3, double *ball2);
 
-/* get_game_state(int_team=HAPPY / GRUMPY) of the current state (RR_Observers.py). */
+/* get_game_state(int_team=HAPPY / GRUMPY) of the current state (RR_Observers.py).  Buffers aligned to out_t. */
 int rr_observe(rr_sim *s, void *obs_h_dev, void *obs_g_dev, void *stream);
 
 /* get_game_state(obj_robot=lstRobots[robot], obj_ball=lstBalls[ball]) of the current state for every env
@@ -174,9 +177,11 @@ int rr_assign_balls(rr_sim *s, const int32_t *robots_host, int32_t n_robots, int
 
 /* step() x k_steps in ONE fused kernel launch; device buffers (layouts above).  Any output
  * pointer may be NULL.  n_actions = values supplied per env per step (robots beyond it keep
- * their thrust, RR_EnvBase.py:272-273).  A discrete action id above 7 (KeyError in the reference, :603-606) leaves the
- * env untouched for that step and raises RR_ERR_BAD_ACTION (done = 1).
- * Alignment: none required.  Result rows are written as coalesced 128-bit stores when a buffer is 16-byte aligned and
+ * their thrust, RR_EnvBase.py:272-273).  A discrete action id above 7 (KeyError in the reference, :603-606), or a
+ * continuous thrust whose round-half-to-even value is not finite or lies outside [-8, 7], leaves the env untouched for
+ * that step and raises RR_ERR_BAD_ACTION (done = 1; with auto_reset the env is reset).
+ * Alignment: every buffer to its element type (out_t results, float actions; RR_E_INVALID otherwise), nothing beyond
+ * that.  Result rows are written as coalesced 128-bit stores when a buffer is 16-byte aligned and
  * its per-step row (N * D * sizeof(out_t), N * 2 * sizeof(out_t), N bytes) is a multiple of 16 bytes, element by
  * element otherwise; discrete actions with n_actions == 4 are read with one 32-bit load per env when the buffer is
  * 4-byte aligned, byte by byte otherwise. */
@@ -229,7 +234,8 @@ int rr_step_host_end(rr_sim *s, int32_t ticket);
 /* Complete physics state, HOST buffers, array-of-structs layout used by the parity harness
  * (oracle/ref_harness.py): rob[N][R][7] = cx,cy,left,right,top,bottom,rot (FloatRect fields,
  * MyUtils.py:122-130); rhist[N][R][3] = pose in history slot count-1 (RR_Robot.py:43-58);
- * rflag[N][R][3] = thrust_l, thrust_r, hist_valid; ball[N][B][8] = cx,cy,l,r,t,b,vx,vy;
+ * rflag[N][R][3] = thrust_l, thrust_r (each in [-8, 7]), hist_valid (0 or 1): rr_set_state returns RR_E_INVALID for
+ * anything else and changes nothing; ball[N][B][8] = cx,cy,l,r,t,b,vx,vy;
  * step[N] = lngStepCount.  These synchronise the device.  rr_set_state also sets what is derived from the injected
  * pose: rectDblPriorStep of every robot and ball (observer RR_OBS_ALLCOORDS_PRIOR) becomes a copy() of the injected
  * rects, as the reference's on_reset / on_step_begin leave it; goal bookkeeping (goal_scoring) restarts as after a

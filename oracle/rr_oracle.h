@@ -60,6 +60,8 @@ extern "C" {
 #define RRO_ERR_UNRESOLVED_FRAME 32u    /* :417-421              */
 #define RRO_ERR_COINCIDENT_BALLS 64u    /* RR_TrashyPhysics.py:249-250 */
 #define RRO_ERR_DIV0 128u               /* MyUtils.py:25         */
+#define RRO_ERR_BAD_ACTION 512u        /* discrete id outside 0..7 (KeyError, RR_EnvBase.py:593-606); NaN or +-inf thrust
+                                           (round() raises, RR_Robot.py:100-102) */
 
 typedef struct {
   int arena_w, arena_h;      /* RR_Constants.py:6-7   */

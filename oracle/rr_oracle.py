@@ -17,7 +17,7 @@ OBS_NONE, OBS_BASIC_LIDAR, OBS_LIDAR6_V2, OBS_ALLCOORDS, OBS_ALLCOORDS_PRIOR, OB
 
 ERR_BITS = {
     1: "STEP_AFTER_DONE", 2: "TOO_MANY_COMMANDS", 4: "BOT_COLLISIONS", 8: "UNDO_FAILED",
-    16: "ROBOTS_STUCK", 32: "UNRESOLVED_FRAME", 64: "COINCIDENT_BALLS", 128: "DIV0",
+    16: "ROBOTS_STUCK", 32: "UNRESOLVED_FRAME", 64: "COINCIDENT_BALLS", 128: "DIV0", 512: "BAD_ACTION",
 }
 
 

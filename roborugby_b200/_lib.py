@@ -27,7 +27,8 @@ ERR_BITS = {
     64: "Really tho?? The balls are in the EXACT same spot????",  # RR_TrashyPhysics.py:250
     128: "Numerator AND Denominator are both 0.",                 # MyUtils.py:25
     256: "reset placement loop exceeded its bound",
-    512: "KeyError: discrete action id outside 0..7",              # RR_EnvBase.py:593-606 (dict lookup)
+    512: "invalid action: a discrete id outside 0..7 (KeyError), or a thrust whose int(round(x)) is NaN, infinite or "
+         "outside [-8, 7]",                                         # RR_EnvBase.py:593-606, RR_Robot.py:100-102
 }
 
 

@@ -283,21 +283,10 @@ __global__ void __launch_bounds__(L::kMaxBlock, L::kStepBlocksPerSM) k_step(cons
 #pragma unroll 1
           for (int r = 0; r < A; r++) w |= (uint32_t)ap[r] << (8 * r);
         }
-#pragma unroll
-        for (int r = 0; r < R; r++) {
-          int l, rt_;
-          const unsigned id = (w >> (8 * r)) & 0xff;
-          bad_action |= r < A && id > 7u;  // KeyError before anything moves (RR_EnvBase.py:593-606, :624)
-          thrust_from_direction((int)id, l, rt_);
-          cmd |= pack_thrust(r, l, rt_);
-        }
+        bad_action = !decode_discrete<R>(w, A, cmd);
       } else {
-        const float *ap = (const float *)a.actions + row * A;
         n_cmd = A / 2;
-#pragma unroll
-        for (int r = 0; r < R; r++)
-          if (r < n_cmd)  // int(round(x)): round half to even (RR_Robot.py:100-102)
-            cmd |= pack_thrust(r, (int)rint((double)ap[2 * r]), (int)rint((double)ap[2 * r + 1]));
+        bad_action = !decode_continuous<R>((const float *)a.actions + row * A, n_cmd, cmd);
       }
     }
     StepOut o;
@@ -931,9 +920,16 @@ int rr_get_starting_positions(rr_sim *s, double *rob3, double *ball2) {
   return RR_OK;
 }
 
+// The kernels store out_t elements and load float actions / int32 ball indices: a pointer that is not aligned to its
+// element type would fault on the device, so the entry points refuse it.
+static bool misaligned(const void *p, size_t align) { return ((uintptr_t)p & (align - 1)) != 0; }
+static size_t out_size(const rr_sim *s) { return s->cfg.out_f64 ? 8 : 4; }
+
 int rr_observe(rr_sim *s, void *obs_h, void *obs_g, void *stream) {
   if (!s) return fail(RR_E_INVALID, "null handle");
   if (rr_obs_dim(s) == 0) return RR_OK;
+  if (misaligned(obs_h, out_size(s)) || misaligned(obs_g, out_size(s)))
+    return fail(RR_E_INVALID, "observation buffers must be aligned to their element type");
   ON_DEVICE(s->device);
   cudaStream_t st = (cudaStream_t)stream;
   if (int jr = join_into(s, st)) return jr;
@@ -954,6 +950,8 @@ int rr_observe_entity(rr_sim *s, int32_t robot, int32_t ball, const int32_t *bal
   if (ob == RR_OBS_NONE) return fail(RR_E_INVALID, "this env has no observer");
   if (robot < 0 || robot >= s->R) return fail(RR_E_INVALID, "robot index out of range");
   if (!ball_dev && ball >= s->B) return fail(RR_E_INVALID, "ball index out of range");
+  if (misaligned(obs, out_size(s)) || misaligned(ball_dev, 4))
+    return fail(RR_E_INVALID, "obs and ball_dev must be aligned to their element types");
   ON_DEVICE(s->device);
   cudaStream_t st = (cudaStream_t)stream;
   if (int jr = join_into(s, st)) return jr;
@@ -1001,12 +999,14 @@ int rr_step(rr_sim *s, const void *actions, int32_t n_actions, int32_t k_steps, 
   int rc = check_actions(s, n_actions, k_steps);
   if (rc) return rc;
   if (n_actions > 0 && !actions) return fail(RR_E_INVALID, "actions is null");
+  const size_t osz = out_size(s);
+  if (misaligned(obs_h, osz) || misaligned(obs_g, osz) || misaligned(rew, osz) || (!s->cfg.discrete && misaligned(actions, 4)))
+    return fail(RR_E_INVALID, "result buffers must be aligned to their element type, continuous actions to 4 bytes");
   ON_DEVICE(s->device);
   cudaStream_t st = (cudaStream_t)stream;
   Consts k = s->k;
   k.n_actions = n_actions;
   // 128-bit result stores need 16-byte aligned buffers whose per-step rows are multiples of 16 bytes
-  const size_t osz = s->cfg.out_f64 ? 8 : 4;
   auto rows16 = [&](const void *p, size_t row_bytes) { return (((uintptr_t)p) & 15u) == 0 && (row_bytes & 15u) == 0; };
   unsigned vec = 0;
   const size_t D = (size_t)rr_obs_dim(s);
@@ -1199,10 +1199,16 @@ int rr_step_host_end(rr_sim *s, int32_t ticket) {
 int rr_set_state(rr_sim *s, const double *rob, const double *rhist, const int32_t *rflag, const double *ball,
                  const int32_t *step) {
   if (!s || !rob || !rhist || !rflag || !ball || !step) return fail(RR_E_INVALID, "null argument");
-  ON_DEVICE(s->device);
-  CK(cudaDeviceSynchronize());
   const int64_t N = s->N;
   const int R = s->R, B = s->B;
+  for (int64_t q = 0; q < N * R; q++) {  // what the packed si column can hold (Env::thrust: 4 bits per thrust)
+    const int32_t *g = rflag + 3 * q;
+    if (g[0] < -8 || g[0] > 7 || g[1] < -8 || g[1] > 7 || (g[2] != 0 && g[2] != 1))
+      return fail(RR_E_INVALID, "rflag of env " + std::to_string(q / R) + " robot " + std::to_string(q % R) +
+                                    ": thrusts must lie in [-8, 7] and hist_valid must be 0 or 1");
+  }
+  ON_DEVICE(s->device);
+  CK(cudaDeviceSynchronize());
   const int NFP = s->NF + prior_columns(s);
   std::vector<double> sf((size_t)NFP * N);
   std::vector<int32_t> si((size_t)s->NI * N);
@@ -1216,7 +1222,7 @@ int rr_set_state(rr_sim *s, const double *rob, const double *rhist, const int32_
       for (int q = 0; q < 3; q++) sf[(size_t)(f + 7 + q) * N + i] = h[q];
       f += 10;
       const int32_t *g = rflag + (i * R + r) * 3;
-      si[(size_t)r * N + i] = (g[0] & 0xff) | ((g[1] & 0xff) << 8) | ((g[2] ? 1 : 0) << 16);
+      si[(size_t)r * N + i] = (g[0] & 0xff) | ((g[1] & 0xff) << 8) | (g[2] << 16);
     }
     for (int b = 0; b < B; b++) {
       const double *p = ball + (i * B + b) * 8;

@@ -63,6 +63,22 @@ static void store(const E &e, double *rob, double *rhist, int32_t *rflag, double
   *step = e.step;
 }
 
+// k_step's action decoding for one env-step of `n` actions given as doubles: discrete ids (the ABI's uint8: 0..255) or
+// thrusts (the ABI's float: rounded to float first).  false: the step is refused (RR_ERR_BAD_ACTION).
+template <int R>
+static bool decode_actions(const Consts &k, const double *a, int n, unsigned &cmd, int &n_cmd) {
+  if (k.discrete) {
+    uint32_t ids = 0;
+    for (int r = 0; r < n && r < R; r++) ids |= ((uint32_t)a[r] & 0xffu) << (8 * r);
+    n_cmd = n;
+    return decode_discrete<R>(ids, n, cmd);
+  }
+  float f[2 * R];
+  for (int q = 0; q < 2 * R; q++) f[q] = q < n ? (float)a[q] : 0.0f;
+  n_cmd = n / 2;
+  return decode_continuous<R>(f, n_cmd, cmd);
+}
+
 static double g_last_replays = 0.0;  // frames of the last emul_step answered by the squeeze memo
 static double g_last_whole = 0.0;    // ... of which whole frames
 static double g_last_stuck = 0.0;    // robot-robot phases answered by the stuck-pair memo
@@ -77,20 +93,10 @@ static unsigned step_t(const Consts &k, double *rob, double *rhist, int32_t *rfl
   load(e, k, rob, rhist, rflag, ball, *step);
   unsigned cmd = 0;
   int n_cmd;
-  if (k.discrete) {
-    n_cmd = n_actions;
-    for (int r = 0; r < n_cmd && r < E::R; r++) {
-      int l, rt;
-      thrust_from_direction((int)actions[r], l, rt);
-      cmd |= pack_thrust(r, l, rt);
-    }
-  } else {
-    n_cmd = n_actions / 2;
-    for (int r = 0; r < n_cmd && r < E::R; r++)
-      cmd |= pack_thrust(r, (int)rint((double)(float)actions[2 * r]), (int)rint((double)(float)actions[2 * r + 1]));
-  }
+  const bool ok = decode_actions<E::R>(k, actions, n_actions, cmd, n_cmd);
   StepOut o;
-  { FrameSync fs_; sim_step(e, k, cmd, n_cmd, o, true, fs_); }
+  { FrameSync fs_; sim_step(e, k, cmd, n_cmd, o, ok, fs_); }
+  if (!ok) o.step_err = RR_ERR_BAD_ACTION;
   g_last_replays = e.mm(kMReplays);
   g_last_whole = e.mm(kMFrames);
   g_last_stuck = e.mm(kMStuckReplays);
@@ -116,16 +122,14 @@ static unsigned step_k_t(const Consts &k, double *rob, double *rhist, int32_t *r
   unsigned errs = 0;
   for (int s = 0; s < K; s++) {
     unsigned cmd = 0;
-    for (int r = 0; r < n_actions && r < E::R; r++) {
-      int l, rt;
-      thrust_from_direction((int)actions[s * n_actions + r], l, rt);
-      cmd |= pack_thrust(r, l, rt);
-    }
+    int n_cmd;
+    const bool ok = decode_actions<E::R>(k, actions + (size_t)s * n_actions, n_actions, cmd, n_cmd);
     StepOut o;
-    { FrameSync fs_; sim_step(e, k, cmd, n_actions, o, true, fs_); }
+    { FrameSync fs_; sim_step(e, k, cmd, n_cmd, o, ok, fs_); }
+    if (!ok) o.step_err = RR_ERR_BAD_ACTION;
     rew_out[2 * s] = o.rew_h; rew_out[2 * s + 1] = o.rew_g;
     errs |= o.step_err;
-    if (o.step_err) break;
+    if (o.step_err & ~RR_ERR_BAD_ACTION) break;  // a refused step leaves the env untouched: k_step goes on from it
   }
   counters[0] = e.mm(kMReplays); counters[1] = e.mm(kMFrames); counters[2] = e.mm(kMStuckReplays);
   store(e, rob, rhist, rflag, ball, step);
@@ -147,21 +151,10 @@ static unsigned goal_rollout_t(const Consts &k, double *rob, double *rhist, int3
   for (int s = 0; s < K; s++) {
     unsigned cmd = 0;
     int n_cmd;
-    const double *a = actions + (size_t)s * stride;
-    if (k.discrete) {
-      n_cmd = n_act[s];
-      for (int r = 0; r < n_cmd && r < E::R; r++) {
-        int l, rt;
-        thrust_from_direction((int)a[r], l, rt);
-        cmd |= pack_thrust(r, l, rt);
-      }
-    } else {
-      n_cmd = n_act[s] / 2;
-      for (int r = 0; r < n_cmd && r < E::R; r++)
-        cmd |= pack_thrust(r, (int)rint((double)(float)a[2 * r]), (int)rint((double)(float)a[2 * r + 1]));
-    }
+    const bool ok = decode_actions<E::R>(k, actions + (size_t)s * stride, n_act[s], cmd, n_cmd);
     StepOut o;
-    { FrameSync fs_; sim_step(e, k, cmd, n_cmd, o, true, fs_); }
+    { FrameSync fs_; sim_step(e, k, cmd, n_cmd, o, ok, fs_); }
+    if (!ok) o.step_err = RR_ERR_BAD_ACTION;
     errs |= o.step_err;
     if (o.step_err) break;
     rew_out[2 * s] = o.rew_h; rew_out[2 * s + 1] = o.rew_g;
