@@ -179,7 +179,11 @@ int rr_assign_balls(rr_sim *s, const int32_t *robots_host, int32_t n_robots, int
  * pointer may be NULL.  n_actions = values supplied per env per step (robots beyond it keep
  * their thrust, RR_EnvBase.py:272-273).  A discrete action id above 7 (KeyError in the reference, :603-606), or a
  * continuous thrust whose round-half-to-even value is not finite or lies outside [-8, 7], leaves the env untouched for
- * that step and raises RR_ERR_BAD_ACTION (done = 1; with auto_reset the env is reset).
+ * that step and raises RR_ERR_BAD_ACTION (done = 1; with auto_reset the env is reset).  A step on a finished env (step
+ * counter above T, or with goal scoring a destroyed goal or no ball left) is refused with RR_ERR_STEP_AFTER_DONE
+ * (done = 1) and changes nothing; continuous actions are not looked at then, as in the reference, while a discrete id
+ * above 7 still raises RR_ERR_BAD_ACTION.  With auto_reset every row that reports done resets the env inside the
+ * launch, a refused one included.  What each row adds to the statistics: rr_get_stats.
  * Alignment: every buffer to its element type (out_t results, float actions; RR_E_INVALID otherwise), nothing beyond
  * that.  Result rows are written as coalesced 128-bit stores when a buffer is 16-byte aligned and
  * its per-step row (N * D * sizeof(out_t), N * 2 * sizeof(out_t), N bytes) is a multiple of 16 bytes, element by
@@ -256,8 +260,21 @@ int rr_error_mask(rr_sim *s, uint32_t *err_host, int32_t clear);
 int rr_last_naughty(rr_sim *s, int32_t *count_host);
 
 /* Episode statistics accumulated on the device since the last rr_clear_stats: RR_NUM_STATS doubles
- * (finished episodes, sum of happy/grumpy returns, sum of lengths, naughty events, errors, steps).
- * rr_stats_device_ptr exposes the device vector so a caller can all-reduce it in place (NCCL). */
+ * (finished episodes, sum of happy/grumpy returns, sum of lengths, naughty events, errors, steps, squeeze replays).
+ * What one row (one env, one env-step) adds:
+ *   steps     1, unless the row is an RR_ERR_STEP_AFTER_DONE refusal
+ *   errors    1 if the row counts as a step and raised (any bit, RR_ERR_BAD_ACTION included)
+ *   naughty   len(set_naughty_bots) of a completed row (what rr_last_naughty reports); 0 on a row that raised and
+ *             without NaughtyBots
+ *   episodes, returns, length
+ *             at the FIRST row that reports done = 1 and is not a refusal since the env's last reset (rr_create,
+ *             rr_reset, rr_reset_fixed, auto-reset) or rr_set_state: 1, the fp64 sum of the rows' rewards since then in
+ *             step order (rows that raised add 0), the step counter.  Later done rows of the same episode (the raw
+ *             row at T + 1 after the TimeLimit row at T, a bad action on a finished env) add nothing here.
+ *   replays   physics frames of the launch answered by the squeeze memo (0 with RR_FLAG_NO_SQUEEZE_MEMO)
+ * Each launch sums its rows per warp and adds them with one fp64 atomic per warp and statistic, so the returns of
+ * a batch differ from a sequential sum in the last bits.  rr_stats_device_ptr exposes the device vector so a caller
+ * can all-reduce it in place (NCCL). */
 int rr_get_stats(rr_sim *s, double *stats_host);
 int rr_stats_device_ptr(rr_sim *s, double **stats_dev);
 int rr_clear_stats(rr_sim *s, void *stream);

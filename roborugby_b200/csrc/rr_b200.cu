@@ -7,7 +7,8 @@
 // HBM layout (DESIGN.md §3): structure of arrays, env index fastest.
 //   sf : double [NF][N]   per robot cx,cy,left,right,top,bottom,rot,hx,hy,hrot ; per ball
 //                         cx,cy,left,right,top,bottom,vx,vy ; episode return happy, grumpy
-//   si : int32  [NI][N]   per robot (thrust_l & 0xff) | (thrust_r & 0xff) << 8 | hist_valid << 16 ;
+//   si : int32  [NI][N]   per robot (thrust_l & 0xff) | (thrust_r & 0xff) << 8 | hist_valid << 16
+//                         (robot 0: | episode counted << 17, rr_sim.cuh pack_robot_word) ;
 //                         step, episode, sticky error mask, naughty count of the last step
 // One thread owns one env for a whole launch: it loads its column of sf/si with coalesced 8-byte /
 // 4-byte transactions, advances k_steps env-steps (12 physics frames each) out of registers / L1,
@@ -113,9 +114,7 @@ __device__ __forceinline__ void load_env(typename L::E &e, double *cold, const C
     for (int q = 0; q < 3; q++) e.rc(r, q) = sf[(f + 7 + q) * N + i];
     e.rc(r, 3) = rr_nan(); e.rc(r, 8) = rr_nan();  // heading-keyed caches start empty
     f += L::kRobotF;
-    int32_t p = si[r * N + i];
-    e.set_thrust(r, (int)(int8_t)(p & 0xff), (int)(int8_t)((p >> 8) & 0xff));
-    e.hvalid |= ((p >> 16) & 1u) << r;
+    unpack_robot_word(e, r, si[r * N + i]);
     robot_refresh_corners(e, k, r);
   }
 #pragma unroll 1
@@ -155,7 +154,7 @@ __device__ __forceinline__ void store_env(const typename L::E &e, const Consts &
 #pragma unroll
     for (int q = 0; q < 3; q++) sf[(f + 7 + q) * N + i] = e.rc(r, q);
     f += L::kRobotF;
-    si[r * N + i] = (e.thl(r) & 0xff) | ((e.thr(r) & 0xff) << 8) | (((e.hvalid >> r) & 1u) << 16);
+    si[r * N + i] = pack_robot_word(e, r);
   }
 #pragma unroll 1
   for (int b = 0; b < L::B; b++) {
@@ -284,7 +283,7 @@ __global__ void __launch_bounds__(L::kMaxBlock, L::kStepBlocksPerSM) k_step(cons
           for (int r = 0; r < A; r++) w |= (uint32_t)ap[r] << (8 * r);
         }
         bad_action = !decode_discrete<R>(w, A, cmd);
-      } else {
+      } else if (decode_before_refusal(e, k)) {
         n_cmd = A / 2;
         bad_action = !decode_continuous<R>((const float *)a.actions + row * A, n_cmd, cmd);
       }
@@ -294,31 +293,8 @@ __global__ void __launch_bounds__(L::kMaxBlock, L::kStepBlocksPerSM) k_step(cons
     fs.parity = (unsigned)s;  // (RR_DETACH is off in diagnostics builds: the field is free)
 #endif
     sim_step(e, k, cmd, n_cmd, o, live && !bad_action, fs);  // (every thread calls it: block-wide barriers inside)
-    if (bad_action) { o.step_err = RR_ERR_BAD_ACTION; e.err |= RR_ERR_BAD_ACTION; }
     int done_flag = 0;
-    if (live) {
-      e.ret_h += o.rew_h; e.ret_g += o.rew_g;
-      last_naughty = rr_popc(o.naughty);
-      const bool aborted = o.step_err != 0;
-      done_flag = (o.done || aborted) ? 1 : 0;
-      // a step refused because the episode is over ("Game is over", :261-262; only without auto_reset) is not an
-      // env-step, not a new error and not another finished episode
-      const bool refused = (o.step_err & RR_ERR_STEP_AFTER_DONE) != 0;
-      if (!refused) {
-        st[RR_STAT_STEPS] += 1.0;
-        st[RR_STAT_NAUGHTY] += (double)last_naughty;
-        if (aborted) st[RR_STAT_ERRORS] += 1.0;
-      }
-      if (done_flag && !refused) {
-        st[RR_STAT_EPISODES] += 1.0;
-        st[RR_STAT_RETURN_HAPPY] += e.ret_h; st[RR_STAT_RETURN_GRUMPY] += e.ret_g;
-        st[RR_STAT_LENGTH] += (double)e.step;
-        if (k.auto_reset) {
-          e.episode += 1;
-          reset_env(e, k, (uint64_t)(k.env_offset + i));
-        }
-      }
-    }
+    if (live) done_flag = step_bookkeeping(e, k, o, bad_action, st, last_naughty, (uint64_t)(k.env_offset + i));
     // Results: written once, never read back by this launch.  Every warp turns its 32 rows of each buffer into
     // coalesced 128-bit streaming stores (warp_store_rows); all lanes of the warp take part (no divergence here).
     {

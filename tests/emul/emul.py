@@ -60,6 +60,17 @@ def lib():
         L.emul_goal_rollout.restype = C.c_uint
         L.emul_step_k.argtypes = [C.POINTER(Config), vp, vp, vp, vp, vp, vp, C.c_int, C.c_int, vp, vp]
         L.emul_step_k.restype = C.c_uint
+        i64 = C.c_int64
+        L.emul_cols_dims.argtypes = [C.POINTER(Config), vp, vp]
+        L.emul_cols_dims.restype = None
+        L.emul_cols_set_state.argtypes = [C.POINTER(Config), vp, vp, i64, i64, vp, vp, vp, vp, C.c_int32]
+        L.emul_cols_set_state.restype = None
+        L.emul_cols_get_state.argtypes = [C.POINTER(Config), vp, vp, i64, i64, vp, vp, vp, vp, vp]
+        L.emul_cols_get_state.restype = None
+        L.emul_cols_reset.argtypes = [C.POINTER(Config), vp, vp, i64, vp, C.c_int]
+        L.emul_cols_reset.restype = None
+        L.emul_launch.argtypes = [C.POINTER(Config), vp, vp, i64, vp, C.c_int, C.c_int] + [vp] * 7
+        L.emul_launch.restype = None
         L.emul_last_replays.argtypes = []
         L.emul_last_replays.restype = C.c_double
         L.emul_last_whole_frames.argtypes = []
@@ -139,6 +150,68 @@ class EmulEnv:
         lib().emul_observe(C.byref(self.cfg), _p(self.rob), _p(self.rhist), _p(self.rflag), _p(self.ball),
                            _p(self.stepc), int(team), _p(o))
         return o[:self.obs_dim]
+
+
+class EmulBatch:
+    """M envs whose complete state persists between calls in the HBM layout of rr_b200.cu (sf [NF][M], si [NI][M]):
+    launch() does what one k_step launch does, with the bookkeeping and auto-reset of the kernel source."""
+
+    def __init__(self, cfg, M, R, B, obs_dim):
+        self.cfg, self.M, self.R, self.B, self.obs_dim = cfg, M, R, B, obs_dim
+        nf = np.zeros(1, np.int32); ni = np.zeros(1, np.int32)
+        lib().emul_cols_dims(C.byref(cfg), _p(nf), _p(ni))
+        self.sf = np.zeros((int(nf[0]), M)); self.si = np.zeros((int(ni[0]), M), np.int32)
+        self.reset(create=True)
+
+    def reset(self, mask=None, create=False):
+        """rr_create (create=True) or rr_reset of the envs whose mask entry is true (None: all)."""
+        m = None if mask is None else np.ascontiguousarray(mask, np.uint8)
+        lib().emul_cols_reset(C.byref(self.cfg), _p(self.sf), _p(self.si), self.M, None if m is None else _p(m),
+                              int(create))
+
+    def set_state(self, i, st):
+        """rr_set_state for env i."""
+        rob = np.ascontiguousarray(st["rob"], np.float64); rhist = np.ascontiguousarray(st["rhist"], np.float64)
+        rflag = np.ascontiguousarray(st["rflag"], np.int32); ball = np.ascontiguousarray(st["ball"], np.float64)
+        lib().emul_cols_set_state(C.byref(self.cfg), _p(self.sf), _p(self.si), self.M, int(i), _p(rob), _p(rhist),
+                                  _p(rflag), _p(ball), int(st["step"]))
+
+    def get_state(self, i):
+        """rr_get_state of env i."""
+        rob = np.zeros((self.R, 7)); rhist = np.zeros((self.R, 3)); rflag = np.zeros((self.R, 3), np.int32)
+        ball = np.zeros((self.B, 8)); step = np.zeros(1, np.int32)
+        lib().emul_cols_get_state(C.byref(self.cfg), _p(self.sf), _p(self.si), self.M, int(i), _p(rob), _p(rhist),
+                                  _p(rflag), _p(ball), _p(step))
+        return dict(rob=rob, rhist=rhist, rflag=rflag, ball=ball, step=np.int32(step[0]))
+
+    @property
+    def episode(self):
+        return self.si[self.R + 1].copy()
+
+    def error_mask(self, clear=False):
+        """rr_error_mask."""
+        m = self.si[self.R + 2].astype(np.uint32)
+        if clear:
+            self.si[self.R + 2] = 0
+        return m
+
+    def last_naughty(self):
+        return self.si[self.R + 3].copy()
+
+    def launch(self, actions, observe=False):
+        """One launch of K steps; actions [K, M, A].  Returns dict(rew [K, M, 2], done, err (the row's error bits),
+        naughty [K, M], obs_h / obs_g [K, M, D] (observe=True), stats [M, RR_NUM_STATS]: each env's contribution)."""
+        a = np.ascontiguousarray(actions, np.float64)
+        K, M, A = a.shape
+        assert M == self.M
+        rew = np.zeros((K, M, 2)); done = np.zeros((K, M), np.int32); err = np.zeros((K, M), np.int32)
+        ng = np.zeros((K, M), np.int32); stats = np.zeros((M, 8))
+        oh = og = None
+        if observe and self.obs_dim:
+            oh = np.full((K, M, self.obs_dim), np.nan); og = np.full((K, M, self.obs_dim), np.nan)
+        lib().emul_launch(C.byref(self.cfg), _p(self.sf), _p(self.si), M, _p(a), A, K, _p(rew), _p(done), _p(err),
+                          _p(ng), None if oh is None else _p(oh), None if og is None else _p(og), _p(stats))
+        return dict(rew=rew, done=done, err=err, naughty=ng, obs_h=oh, obs_g=og, stats=stats)
 
 
 def observe_entity(cfg, st, robot, ball, obs_dim):
