@@ -50,7 +50,13 @@ extern "C" {
  * first, 0 ends.  Each on_step_end calls super() before adding its own terms, so the bodies run in REVERSE MRO
  * order, and NaughtyBots.on_step_end does not call super(): mixins listed after it in the class never run.
  * reward_order == 0 selects Naughty, Chase, PushPos, PushNeg, BaseDestruction, DontDrive, KeepMoving (those in the
- * mask), which is the order of the registered ids (RR_Environments.py:11-37). */
+ * mask), which is the order of the registered ids (RR_Environments.py:11-37).
+ * Valid pairs are exactly those a class `class Env(*mixins, Observer, GameEnv_Simple)` with distinct mixins produces:
+ * reward_mask has no bits above RR_REW_PUSHNEG, and reward_order is 0 or all of
+ *   - its nibbles are distinct ids 1..7, each with its bit in reward_mask, and no non-zero nibble follows the first 0;
+ *   - if NAUGHTY is in the mask, the first (lowest) nibble is RR_MIX_NAUGHTY;
+ *   - if NAUGHTY is not in the mask, the order lists exactly the mask's mixins.
+ * rr_create and rr_check_config refuse any other pair with RR_E_INVALID (rr_sim.cuh rr_reward_config_error). */
 #define RR_MIX_CHASE 1u
 #define RR_MIX_PUSHPOS 2u
 #define RR_MIX_NAUGHTY 3u
@@ -133,7 +139,13 @@ typedef struct rr_sim rr_sim;
  * "RoboRugby-v0", "RoboRugbySimple-v0", "RoboRugbySimpleDuel-v2", "RoboRugbySimpleDuel-v3". */
 int rr_default_config(rr_config *cfg, int preset, const char *env_id);
 
-/* GameEnv.__init__ (RR_EnvBase.py:70-123) for n_envs episodes on CUDA device `device`. */
+/* The checks rr_create makes on cfg, without a device: abi_version, preset, observer; discrete, time_limit, auto_reset,
+ * out_f64, strict_reset and goal_scoring are 0 or 1; flags has no unknown bits; env_offset >= 0; (reward_mask,
+ * reward_order) is a valid pair (see RR_MIX_*).  RR_E_INVALID with a message naming the field otherwise. */
+int rr_check_config(const rr_config *cfg);
+
+/* GameEnv.__init__ (RR_EnvBase.py:70-123) for n_envs episodes on CUDA device `device`.  cfg is checked
+ * (rr_check_config) before any device is looked at. */
 int rr_create(const rr_config *cfg, int64_t n_envs, int device, rr_sim **out);
 int rr_destroy(rr_sim *s);
 const char *rr_last_error(void);

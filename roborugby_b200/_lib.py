@@ -47,6 +47,7 @@ class Config(C.Structure):
 _vp, _i32, _i64 = C.c_void_p, C.c_int32, C.c_int64
 SIGNATURES = {
     "rr_default_config": (C.c_int, [C.POINTER(Config), C.c_int, C.c_char_p]),
+    "rr_check_config": (C.c_int, [C.POINTER(Config)]),
     "rr_create": (C.c_int, [C.POINTER(Config), _i64, C.c_int, C.POINTER(_vp)]),
     "rr_destroy": (C.c_int, [_vp]),
     "rr_last_error": (C.c_char_p, []),
@@ -108,6 +109,12 @@ def load():
 def check(rc):
     if rc != 0:
         raise RRError(load().rr_last_error().decode() or f"rr error {rc}")
+
+
+def check_config(cfg):
+    """rr_check_config: ValueError naming the field if rr_create would refuse cfg."""
+    if load().rr_check_config(C.byref(cfg)) != 0:
+        raise ValueError(load().rr_last_error().decode())
 
 
 def default_config(preset, env_id):

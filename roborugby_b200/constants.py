@@ -78,6 +78,8 @@ def reward_config_from_mixins(mixins):
     for name in mixins:
         if name not in REWARD_MIXINS:
             raise ValueError(f"unknown reward mixin {name!r}; expected one of {sorted(REWARD_MIXINS)}")
+        if mask & REWARD_MIXINS[name][0]:   # Python refuses such a class: "duplicate base class"
+            raise ValueError(f"reward mixin {name!r} listed twice")
         mask |= REWARD_MIXINS[name][0]
     for name in mixins:           # MRO order; the chain of super() calls stops at NaughtyBots
         chain.append(name)
@@ -86,6 +88,4 @@ def reward_config_from_mixins(mixins):
     order = 0
     for n, name in enumerate(reversed(chain)):
         order |= REWARD_MIXINS[name][1] << (4 * n)
-    if len(chain) > 8:
-        raise ValueError("at most 8 mixins")
     return mask, order

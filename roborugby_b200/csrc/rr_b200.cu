@@ -629,11 +629,30 @@ static inline int prior_columns(const rr_sim *s) {
   return s->cfg.observer == RR_OBS_ALLCOORDS_PRIOR ? 3 * s->R + 2 * s->B : 0;
 }
 
-int rr_create(const rr_config *cfg, int64_t n_envs, int device, rr_sim **out) {
-  if (!cfg || !out || n_envs <= 0) return fail(RR_E_INVALID, "bad arguments");
+int rr_check_config(const rr_config *cfg) {
+  if (!cfg) return fail(RR_E_INVALID, "null argument");
   if (cfg->abi_version != RR_ABI_VERSION) return fail(RR_E_INVALID, "abi_version mismatch");
   if (cfg->preset != RR_PRESET_GAME && cfg->preset != RR_PRESET_TRAIN) return fail(RR_E_INVALID, "unknown preset");
   if (cfg->observer < 0 || cfg->observer > RR_OBS_LIDAR6_V1) return fail(RR_E_INVALID, "unknown observer");
+  const struct { const char *name; int32_t v; } bools[] = {
+      {"discrete", cfg->discrete},     {"time_limit", cfg->time_limit},     {"auto_reset", cfg->auto_reset},
+      {"out_f64", cfg->out_f64},       {"strict_reset", cfg->strict_reset}, {"goal_scoring", cfg->goal_scoring}};
+  for (const auto &b : bools)
+    if (b.v != 0 && b.v != 1) return fail(RR_E_INVALID, std::string(b.name) + " must be 0 or 1, got " + std::to_string(b.v));
+  if (cfg->flags & ~RR_FLAG_NO_SQUEEZE_MEMO)
+    return fail(RR_E_INVALID, "flags has unknown bits " + std::to_string(cfg->flags & ~RR_FLAG_NO_SQUEEZE_MEMO));
+  if (cfg->env_offset < 0) return fail(RR_E_INVALID, "env_offset must be >= 0");
+  if (const char *why = rr_reward_config_error(cfg->reward_mask, cfg->reward_order)) {
+    char hex[48];
+    snprintf(hex, sizeof hex, " (reward_mask 0x%x, reward_order 0x%x)", cfg->reward_mask, cfg->reward_order);
+    return fail(RR_E_INVALID, std::string(why) + hex);
+  }
+  return RR_OK;
+}
+
+int rr_create(const rr_config *cfg, int64_t n_envs, int device, rr_sim **out) {
+  if (!cfg || !out || n_envs <= 0) return fail(RR_E_INVALID, "bad arguments");
+  if (const int rc = rr_check_config(cfg)) return rc;
   int ndev = 0;
   cudaError_t ce = cudaGetDeviceCount(&ndev);
   if (ce != cudaSuccess || ndev == 0)

@@ -29,8 +29,6 @@ class RoboRugbyVecEnv:
                  goal_scoring=False, pipeline=1):
         if env_id not in ENV_IDS:
             raise ValueError(f"unknown env id {env_id!r}; expected one of {ENV_IDS}")
-        if not torch.cuda.is_available():
-            raise RuntimeError("RoboRugbyVecEnv needs a CUDA device: roborugby_b200 has no CPU fallback")
         self.lib = _lib.load()
         self.env_id = env_id
         self.preset = get_preset(preset)
@@ -58,6 +56,9 @@ class RoboRugbyVecEnv:
         cfg.goal_scoring = int(bool(goal_scoring))   # goal scoring as intended (include/rr_b200.h); default: the reference's HEAD
         cfg.seed = int(seed) & 0xFFFFFFFFFFFFFFFF
         cfg.env_offset = int(env_offset)
+        _lib.check_config(cfg)   # ValueError for a reward_mask / reward_order no class composition produces, etc.
+        if not torch.cuda.is_available():
+            raise RuntimeError("RoboRugbyVecEnv needs a CUDA device: roborugby_b200 has no CPU fallback")
         self.cfg = cfg
         self.out_dtype = torch.float64 if cfg.out_f64 else torch.float32
         self.discrete = bool(cfg.discrete)

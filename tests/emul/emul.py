@@ -71,6 +71,8 @@ def lib():
         L.emul_cols_reset.restype = None
         L.emul_launch.argtypes = [C.POINTER(Config), vp, vp, i64, vp, C.c_int, C.c_int] + [vp] * 7
         L.emul_launch.restype = None
+        L.emul_reward_config_valid.argtypes = [vp, vp, i64, vp]
+        L.emul_reward_config_valid.restype = None
         L.emul_last_replays.argtypes = []
         L.emul_last_replays.restype = C.c_double
         L.emul_last_whole_frames.argtypes = []
@@ -240,6 +242,15 @@ def predicates(cfg, st):
     rr = np.zeros(6, np.int32); br = np.zeros(32, np.int32)
     lib().emul_predicates(C.byref(cfg), _p(rob), _p(rhist), _p(rflag), _p(ball), _p(step), _p(rr), _p(br))
     return rr, br
+
+
+def reward_config_valid(mask, order):
+    """rr_reward_config_valid (rr_sim.cuh) element-wise over two integer arrays -> bool array."""
+    m = np.ascontiguousarray(mask, np.uint32).reshape(-1); o = np.ascontiguousarray(order, np.uint32).reshape(-1)
+    assert m.shape == o.shape
+    ok = np.zeros(m.size, np.uint8)
+    lib().emul_reward_config_valid(_p(m), _p(o), m.size, _p(ok))
+    return ok.astype(bool)
 
 
 def sincos(x, dd_only=False):

@@ -419,6 +419,11 @@ void emul_launch(const rr_config *cfg, double *sf, int32_t *si, int64_t M, const
   EMUL_DISPATCH(cfg, launch_dispatch_t, k, sf, si, M, actions, n_actions, K, rew, done, err, naughty, obs_h, obs_g, stats);
 }
 
+// rr_reward_config_valid over n (mask, order) pairs: ok[i] = 1 for a pair rr_create accepts
+void emul_reward_config_valid(const uint32_t *mask, const uint32_t *order, int64_t n, uint8_t *ok) {
+  for (int64_t i = 0; i < n; i++) ok[i] = rr_reward_config_valid(mask[i], order[i]) ? 1 : 0;
+}
+
 double emul_last_replays(void) { return g_last_replays; }
 double emul_last_whole_frames(void) { return g_last_whole; }
 double emul_last_stuck_replays(void) { return g_last_stuck; }

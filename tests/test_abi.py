@@ -73,6 +73,8 @@ def test_reward_mixin_composition_to_config():
     import pytest
     with pytest.raises(ValueError):
         f(["NoSuchMixin"])
+    with pytest.raises(ValueError):   # "duplicate base class" in Python
+        f(["ChasePosBall", "ChasePosBall"])
 
 
 def test_bench_reference_arm_prints_the_contract_line():
