@@ -204,6 +204,33 @@ int rr_assign_balls(rr_sim *s, const int32_t *robots_host, int32_t n_robots, int
 int rr_step(rr_sim *s, const void *actions_dev, int32_t n_actions, int32_t k_steps, void *obs_h_dev,
             void *obs_g_dev, void *rew_dev, uint8_t *done_dev, void *stream);
 
+/* row_flags bits (rr_step_info) */
+#define RR_ROW_TRUNCATED 1u /* gym 0.17's info['TimeLimit.truncated'] */
+#define RR_ROW_RAISED 2u    /* the row's own error bits are non-zero (the reference raised) */
+
+/* rr_step plus what a learner needs at every episode end, which auto_reset otherwise overwrites inside the launch
+ * (rr_step is this call with three NULLs).  All three outputs are optional device buffers:
+ *   final_obs_h / final_obs_g  out_t [K][N][D]: for every row with done = 1, get_game_state(int_team=HAPPY / GRUMPY) of
+ *     the state the row's step ended in, before any auto-reset: what obs_h / obs_g would hold for that row with
+ *     auto_reset = 0 (so with auto_reset = 0 the done rows equal the obs rows bit for bit).  A row that raised reports the
+ *     state as the kernel left it (what rr_observe reports after it with auto_reset = 0).  Rows with done = 0 are NOT
+ *     written: the caller's memory there is left as it was.  Ignored when D = 0 (RR_OBS_NONE).
+ *   row_flags  uint8 [K][N], written for every row:
+ *     RR_ROW_TRUNCATED  time_limit && step >= T && !game_is_done() on a row that did not raise: the episode was cut by
+ *                       the TimeLimit wrapper (gym_env.py restates the rule for one env).  A goal destroyed at step T
+ *                       is not truncated, neither is the raw row at T + 1 without auto_reset;
+ *     RR_ROW_RAISED     the row's own error bits are non-zero (any RR_ERR_*, RR_ERR_BAD_ACTION and
+ *                       RR_ERR_STEP_AFTER_DONE included): the reference's step() raised;
+ *     other bits 0.  A done row with neither bit is a real end of the episode (terminated).
+ * Everything else (obs, rew and done rows, the state, the error masks, the statistics) is what rr_step computes.  The
+ * checks are rr_step's; final observation buffers must be aligned to out_t as well (RR_E_INVALID, nothing launched).
+ * row_flags rows are written as 128-bit stores when the buffer is 16-byte aligned and N is a multiple of 16.  With a
+ * sub-batch pipeline (rr_set_pipeline) these buffers follow the rule of the others: join before reading them.
+ * rr_step_host and rr_step_host_begin do not report these outputs. */
+int rr_step_info(rr_sim *s, const void *actions_dev, int32_t n_actions, int32_t k_steps, void *obs_h_dev,
+                 void *obs_g_dev, void *rew_dev, uint8_t *done_dev, void *final_obs_h_dev, void *final_obs_g_dev,
+                 uint8_t *row_flags_dev, void *stream);
+
 /* Same call with HOST buffers: copies actions host->device, launches, and synchronises the stream before returning.
  * This is what a single-process caller of the reference's env.step() would bind.  When every result buffer is pinned
  * (page-locked, e.g. cudaHostAlloc / torch pin_memory) the kernel writes its rows straight into host memory (zero

@@ -16,6 +16,7 @@ OBS_NONE, OBS_BASIC_LIDAR, OBS_LIDAR6_V2, OBS_ALLCOORDS, OBS_ALLCOORDS_PRIOR, OB
 NUM_STATS = 8
 STAT_NAMES = ("episodes", "return_happy", "return_grumpy", "length", "naughty", "errors", "steps", "squeeze_replays")
 FLAG_NO_SQUEEZE_MEMO = 1
+ROW_TRUNCATED, ROW_RAISED = 1, 2   # rr_step_info row_flags
 
 ERR_BITS = {
     1: "Game is over. Go home.",                                   # RR_EnvBase.py:262
@@ -64,6 +65,7 @@ SIGNATURES = {
     "rr_observe_entity": (C.c_int, [_vp, _i32, _i32, _vp, _vp, _vp]),
     "rr_assign_balls": (C.c_int, [_vp, _vp, _i32, _vp, _vp]),
     "rr_step": (C.c_int, [_vp, _vp, _i32, _i32, _vp, _vp, _vp, _vp, _vp]),
+    "rr_step_info": (C.c_int, [_vp, _vp, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "rr_step_host": (C.c_int, [_vp, _vp, _i32, _i32, _vp, _vp, _vp, _vp, _vp]),
     "rr_set_pipeline": (C.c_int, [_vp, _i32]),
     "rr_join": (C.c_int, [_vp, _vp]),

@@ -223,9 +223,11 @@ struct StepArgs {
   uint8_t *done;
   int64_t N;
   int K;
-  unsigned vec;  // bit 0 observations, 1 rewards, 2 done: the buffer's rows can be written with 128-bit stores;
-                 // bit 3: the action buffer is 4-byte aligned (one 32-bit load per env when A == 4)
+  unsigned vec;  // bit 0 observations, 1 rewards, 2 done, 4 row_flags: the buffer's rows can be written with 128-bit
+                 // stores; bit 3: the action buffer is 4-byte aligned (one 32-bit load per env when A == 4)
   int block0;    // first block of this launch's env range (sub-batch launches, rr_set_pipeline); 0 for a whole batch
+  void *final_obs_h, *final_obs_g;  // rr_step_info: out_t [K][N][D], written on done rows only (k_step<L, OutT, true>)
+  uint8_t *row_flags;               // rr_step_info: RR_ROW_* [K][N]
 };
 
 __device__ __forceinline__ double warp_sum(double v) {
@@ -236,7 +238,9 @@ __device__ __forceinline__ double warp_sum(double v) {
 
 // The fused multi-step kernel: K env-steps per launch, auto-reset inside.  Padding threads of the
 // last block (i >= N) run the control flow without an env so that the per-frame barrier is uniform.
-template <class L, typename OutT>
+// INFO: also report every row's RR_ROW_* flags and, on done rows, the terminal observation taken before the auto-reset
+// (rr_step_info).  A template switch, not a run-time branch: the default kernels keep their registers and stack.
+template <class L, typename OutT, bool INFO = false>
 __global__ void __launch_bounds__(L::kMaxBlock, L::kStepBlocksPerSM) k_step(const __grid_constant__ Consts k, const __grid_constant__ StepArgs a) {
   using E = typename L::E;
   constexpr int R = E::R;
@@ -294,7 +298,26 @@ __global__ void __launch_bounds__(L::kMaxBlock, L::kStepBlocksPerSM) k_step(cons
 #endif
     sim_step(e, k, cmd, n_cmd, o, live && !bad_action, fs);  // (every thread calls it: block-wide barriers inside)
     int done_flag = 0;
-    if (live) done_flag = step_bookkeeping(e, k, o, bad_action, st, last_naughty, (uint64_t)(k.env_offset + i));
+    if (live) done_flag = step_accounting(e, k, o, bad_action, st, last_naughty);
+    unsigned char row_flag = 0;
+    if constexpr (INFO) {
+      if (live) row_flag = (unsigned char)step_row_flags(e, k, o);
+      // the terminal observation, before the auto-reset: done rows are rare (GAME 1 / 4500 env-steps), so each done lane
+      // observes and stores its own row, without staging
+      if (dim > 0 && (a.final_obs_h || a.final_obs_g)) {
+        const int lane = threadIdx.x & 31;
+        double ob[kMaxObs];
+        unsigned oerr = 0;
+#pragma unroll 1
+        for (int team = 1; team >= -1; team -= 2) {
+          OutT *dst = (OutT *)(team > 0 ? a.final_obs_h : a.final_obs_g);
+          if (!dst) continue;
+          if (live && done_flag) observe(e, k, team, ob, oerr);
+          warp_store_rows<OutT>(dst + (row - lane) * dim, ob, dim, live && done_flag, false, nullptr, lane);
+        }
+      }
+    }
+    if (live) step_auto_reset(e, k, done_flag, (uint64_t)(k.env_offset + i));
     // Results: written once, never read back by this launch.  Every warp turns its 32 rows of each buffer into
     // coalesced 128-bit streaming stores (warp_store_rows); all lanes of the warp take part (no divergence here).
     {
@@ -309,6 +332,12 @@ __global__ void __launch_bounds__(L::kMaxBlock, L::kStepBlocksPerSM) k_step(cons
       if (a.done) {
         const unsigned char dn[1] = {(unsigned char)done_flag};
         warp_store_rows<unsigned char>(a.done + row0, dn, 1, live, full && (a.vec & 4u), stage, lane);
+      }
+      if constexpr (INFO) {
+        if (a.row_flags) {
+          const unsigned char rf[1] = {row_flag};
+          warp_store_rows<unsigned char>(a.row_flags + row0, rf, 1, live, full && (a.vec & 16u), stage, lane);
+        }
       }
       if (dim > 0 && (a.obs_h || a.obs_g)) {
         double ob[kMaxObs];
@@ -601,7 +630,8 @@ static cudaError_t opt_in_shared_memory() {
     cudaError_t r = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
     if (e == cudaSuccess) e = r;
   };
-  set(k_step<L, float>); set(k_step<L, double>); set(k_init<L>); set(k_reset<L>); set(k_reset_fixed<L>);
+  set(k_step<L, float>); set(k_step<L, double>); set(k_step<L, float, true>); set(k_step<L, double, true>);
+  set(k_init<L>); set(k_reset<L>); set(k_reset_fixed<L>);
   set(k_observe<L, float>); set(k_observe<L, double>);
   set(k_observe_entity<L, float>); set(k_observe_entity<L, double>); set(k_assign_balls<L>);
   return e;
@@ -685,11 +715,18 @@ int rr_create(const rr_config *cfg, int64_t n_envs, int device, rr_sim **out) {
   s->stats = s->own_stats;
   if (game) {  // the wide k_step variants
     const int wb = (int)LGameWide::smem_bytes(LGameWide::kMaxBlock);
-    cudaError_t we = cfg->goal_scoring
-        ? (cudaFuncSetAttribute(k_step<LGameGoalsWide, float>, cudaFuncAttributeMaxDynamicSharedMemorySize, wb),
-           cudaFuncSetAttribute(k_step<LGameGoalsWide, double>, cudaFuncAttributeMaxDynamicSharedMemorySize, wb))
-        : (cudaFuncSetAttribute(k_step<LGameWide, float>, cudaFuncAttributeMaxDynamicSharedMemorySize, wb),
-           cudaFuncSetAttribute(k_step<LGameWide, double>, cudaFuncAttributeMaxDynamicSharedMemorySize, wb));
+    cudaError_t we = cudaSuccess;
+    auto set = [&](auto kern) {
+      cudaError_t r = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, wb);
+      if (we == cudaSuccess) we = r;
+    };
+    if (cfg->goal_scoring) {
+      set(k_step<LGameGoalsWide, float>); set(k_step<LGameGoalsWide, double>);
+      set(k_step<LGameGoalsWide, float, true>); set(k_step<LGameGoalsWide, double, true>);
+    } else {
+      set(k_step<LGameWide, float>); set(k_step<LGameWide, double>);
+      set(k_step<LGameWide, float, true>); set(k_step<LGameWide, double, true>);
+    }
     if (we != cudaSuccess) { rr_destroy(s); return fail(RR_E_CUDA, std::string("cudaFuncSetAttribute: ") + cudaGetErrorString(we)); }
   }
   {
@@ -990,6 +1027,11 @@ static int check_actions(const rr_sim *s, int32_t n_actions, int32_t k_steps) {
 
 int rr_step(rr_sim *s, const void *actions, int32_t n_actions, int32_t k_steps, void *obs_h, void *obs_g, void *rew,
             uint8_t *done, void *stream) {
+  return rr_step_info(s, actions, n_actions, k_steps, obs_h, obs_g, rew, done, nullptr, nullptr, nullptr, stream);
+}
+
+int rr_step_info(rr_sim *s, const void *actions, int32_t n_actions, int32_t k_steps, void *obs_h, void *obs_g, void *rew,
+                 uint8_t *done, void *final_obs_h, void *final_obs_g, uint8_t *row_flags, void *stream) {
   if (!s) return fail(RR_E_INVALID, "null handle");
   int rc = check_actions(s, n_actions, k_steps);
   if (rc) return rc;
@@ -997,6 +1039,10 @@ int rr_step(rr_sim *s, const void *actions, int32_t n_actions, int32_t k_steps, 
   const size_t osz = out_size(s);
   if (misaligned(obs_h, osz) || misaligned(obs_g, osz) || misaligned(rew, osz) || (!s->cfg.discrete && misaligned(actions, 4)))
     return fail(RR_E_INVALID, "result buffers must be aligned to their element type, continuous actions to 4 bytes");
+  if (rr_obs_dim(s) == 0) final_obs_h = final_obs_g = nullptr;  // no observation: nothing to report
+  if (misaligned(final_obs_h, osz) || misaligned(final_obs_g, osz))
+    return fail(RR_E_INVALID, "final observation buffers must be aligned to their element type");
+  const bool info = final_obs_h || final_obs_g || row_flags;
   ON_DEVICE(s->device);
   cudaStream_t st = (cudaStream_t)stream;
   Consts k = s->k;
@@ -1009,7 +1055,8 @@ int rr_step(rr_sim *s, const void *actions, int32_t n_actions, int32_t k_steps, 
   if (rows16(rew, s->N * 2 * osz)) vec |= 2u;
   if (rows16(done, (size_t)s->N)) vec |= 4u;
   if ((((uintptr_t)actions) & 3u) == 0) vec |= 8u;
-  StepArgs a{s->sf, s->si, s->stats, actions, obs_h, obs_g, rew, done, s->N, k_steps, vec, 0};
+  if (rows16(row_flags, (size_t)s->N)) vec |= 16u;
+  StepArgs a{s->sf, s->si, s->stats, actions, obs_h, obs_g, rew, done, s->N, k_steps, vec, 0, final_obs_h, final_obs_g, row_flags};
   const bool game = s->cfg.preset == RR_PRESET_GAME, goals = s->cfg.goal_scoring != 0, f64 = s->cfg.out_f64 != 0;
   // one stream-ordered launch per call over more envs than 384-thread blocks cover in one wave: 448-thread blocks
   const bool wide = game && s->pipe <= 1 && (s->N + LGame::kMaxBlock - 1) / LGame::kMaxBlock > s->sms &&
@@ -1020,8 +1067,11 @@ int rr_step(rr_sim *s, const void *actions, int32_t n_actions, int32_t k_steps, 
     a.block0 = block0;
 #define RR_STEP_CASE(LTYPE)                                                                                  \
     do {                                                                                                     \
-      if (f64) k_step<LTYPE, double><<<(unsigned)nblocks, blk, LTYPE::smem_bytes(blk), on>>>(k, a);          \
-      else k_step<LTYPE, float><<<(unsigned)nblocks, blk, LTYPE::smem_bytes(blk), on>>>(k, a);               \
+      const size_t sm = LTYPE::smem_bytes(blk);                                                              \
+      if (info && f64) k_step<LTYPE, double, true><<<(unsigned)nblocks, blk, sm, on>>>(k, a);                \
+      else if (info) k_step<LTYPE, float, true><<<(unsigned)nblocks, blk, sm, on>>>(k, a);                   \
+      else if (f64) k_step<LTYPE, double><<<(unsigned)nblocks, blk, sm, on>>>(k, a);                         \
+      else k_step<LTYPE, float><<<(unsigned)nblocks, blk, sm, on>>>(k, a);                                   \
     } while (0)
     if (game && !goals) { if (wide) RR_STEP_CASE(LGameWide); else RR_STEP_CASE(LGame); }
     else if (!game && !goals) RR_STEP_CASE(LTrain);

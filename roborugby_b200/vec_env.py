@@ -209,25 +209,53 @@ class RoboRugbyVecEnv:
         _lib.check(self.lib.rr_assign_balls(self._h, r.ctypes.data_as(C.c_void_p), len(r), out.data_ptr(), self._stream()))
         return out
 
-    def step(self, actions):
-        """One env-step for all envs.  actions: uint8 [N, A] (discrete ids) or float32 [N, A]."""
-        obs_h, obs_g, rew, done = self.step_k(actions, 1)
+    def step(self, actions, final_info=False):
+        """One env-step for all envs.  actions: uint8 [N, A] (discrete ids) or float32 [N, A].  final_info=True adds to
+        info what auto-reset would otherwise hide (see step_k): "final_observation" / "final_observation_grumpy" [N, D]
+        (valid where done), "TimeLimit.truncated" and "raised" (bool [N])."""
+        out = self.step_k(actions, 1, final_info=final_info)
+        obs_h, obs_g, rew, done = out[:4]
         info = {"obs_grumpy": obs_g[0], "reward_grumpy": rew[0, :, 1]}
+        if final_info:
+            f = out[4]
+            info.update({"final_observation": f["final_obs"][0], "final_observation_grumpy": f["final_obs_grumpy"][0],
+                         "TimeLimit.truncated": f["truncated"][0], "raised": f["raised"][0]})
         return obs_h[0], rew[0, :, 0], done[0].bool(), info
 
-    def step_k(self, actions, k, join=True):
+    def _final_out(self, k):
+        """Persistent rr_step_info buffers for k fused steps."""
+        key = ("final", k)
+        if key not in self._bufs:
+            N, D = self.num_envs, max(self.obs_dim, 1)
+            mk = lambda *s, dt=self.out_dtype: torch.empty(*s, dtype=dt, device=self.device)
+            self._bufs[key] = dict(final_obs_h=mk(k, N, D), final_obs_g=mk(k, N, D), row_flags=mk(k, N, dt=torch.uint8))
+        return self._bufs[key]
+
+    def step_k(self, actions, k, join=True, final_info=False):
         """k fused env-steps in ONE kernel launch (one per group with a sub-batch pipeline).  actions [k, N, A]; returns
         obs_h [k,N,D], obs_g, rew [k,N,2], done [k,N] (uint8).  Envs that finish are reset inside the launch (auto_reset).
         join=False (pipeline > 1 only): do not make the current stream wait for the launches; the caller joins later and
-        must not touch `actions` or the returned buffers before that."""
+        must not touch `actions` or the returned buffers before that.
+        final_info=True (rr_step_info) returns a fifth element, a dict: "final_obs" / "final_obs_grumpy" [k, N, D], the
+        observation of the state each done row ended in, before the auto-reset (rows with done == 0 hold whatever an earlier
+        call left there); "row_flags" [k, N] (uint8, _lib.ROW_TRUNCATED | _lib.ROW_RAISED); "truncated" and "raised" (bool
+        [k, N]): gym's info['TimeLimit.truncated'] and "the reference's step() raised".  A done row with neither is a real
+        end of the episode.  The three buffers persist like the others and, with join=False, follow the same rule; since
+        "truncated" and "raised" are computed from row_flags on the current stream, with join=False they are None: derive
+        them from row_flags after join()."""
         actions = self._check_actions(actions, k)
         A = actions.shape[2]
         b = self._out(k)
         has_obs = self.obs_dim > 0
-        _lib.check(self.lib.rr_step(self._h, actions.data_ptr(), A, k,
-                                    b["obs_h"].data_ptr() if has_obs else None,
-                                    b["obs_g"].data_ptr() if has_obs else None,
-                                    b["rew"].data_ptr(), b["done"].data_ptr(), self._stream()))
+        f = self._final_out(k) if final_info else None
+        _lib.check(self.lib.rr_step_info(self._h, actions.data_ptr(), A, k,
+                                         b["obs_h"].data_ptr() if has_obs else None,
+                                         b["obs_g"].data_ptr() if has_obs else None,
+                                         b["rew"].data_ptr(), b["done"].data_ptr(),
+                                         f["final_obs_h"].data_ptr() if f and has_obs else None,
+                                         f["final_obs_g"].data_ptr() if f and has_obs else None,
+                                         f["row_flags"].data_ptr() if f else None, self._stream()))
+        joined = True
         if self.pipeline > 1:
             if join:
                 self.join()
@@ -235,9 +263,17 @@ class RoboRugbyVecEnv:
                 # keep every action buffer alive until the groups have read it: the groups run on the handle's own streams,
                 # which torch's stream-ordered allocator knows nothing about
                 self._inflight.append(actions)
+                joined = False
                 if len(self._inflight) > 256:   # a caller that never joins: bound what is kept alive
                     self.join()
-        return b["obs_h"][..., :self.obs_dim], b["obs_g"][..., :self.obs_dim], b["rew"], b["done"]
+        out = (b["obs_h"][..., :self.obs_dim], b["obs_g"][..., :self.obs_dim], b["rew"], b["done"])
+        if not final_info:
+            return out
+        fl = f["row_flags"]
+        info = dict(final_obs=f["final_obs_h"][..., :self.obs_dim], final_obs_grumpy=f["final_obs_g"][..., :self.obs_dim],
+                    row_flags=fl, truncated=(fl & _lib.ROW_TRUNCATED).bool() if joined else None,
+                    raised=(fl & _lib.ROW_RAISED).bool() if joined else None)
+        return out + (info,)
 
     def step_host(self, actions_host, k, out=None):
         """Same as step_k through the HOST-buffer entry point rr_step_host: `actions_host` is a pinned
