@@ -4,12 +4,8 @@
 //   nvcc -O3 -std=c++17 -gencode arch=compute_100a,code=sm_100a -lineinfo --fmad=false
 //        -Xcompiler -fPIC -shared -o roborugby_b200/librr_b200.so roborugby_b200/csrc/rr_b200.cu
 //
-// HBM layout (DESIGN.md §3): structure of arrays, env index fastest.
-//   sf : double [NF][N]   per robot cx,cy,left,right,top,bottom,rot,hx,hy,hrot ; per ball
-//                         cx,cy,left,right,top,bottom,vx,vy ; episode return happy, grumpy
-//   si : int32  [NI][N]   per robot (thrust_l & 0xff) | (thrust_r & 0xff) << 8 | hist_valid << 16
-//                         (robot 0: | episode counted << 17, rr_sim.cuh pack_robot_word) ;
-//                         step, episode, sticky error mask, naughty count of the last step
+// HBM layout (DESIGN.md §3): structure of arrays sf (double) and si (int32), env index fastest; the columns are
+// defined once, by rr::Columns in rr_sim.cuh.
 // One thread owns one env for a whole launch: it loads its column of sf/si with coalesced 8-byte /
 // 4-byte transactions, advances k_steps env-steps (12 physics frames each) out of registers / L1,
 // streams actions in and observations, rewards and done flags out per step, and writes the column
@@ -62,13 +58,6 @@ struct Launch {
   static constexpr size_t smem_bytes(int block) {
     return sizeof(double) * (kTrigDoubles + E::kDoubles * (size_t)block) + (size_t)kStageBytes * (block / 32);
   }
-  // HBM structure-of-arrays layout
-  static constexpr int kRobotF = 10, kBallF = 8;
-  // + the rectDblPriorStep poses (3 per robot, 2 per ball) behind the episode returns: allocated always, loaded and
-  // stored only by handles whose observer reports them (RR_OBS_ALLCOORDS_PRIOR)
-  static constexpr int NF_BASE = R * kRobotF + B * kBallF + 2;
-  static constexpr int NF = NF_BASE + 3 * R + 2 * B;
-  static constexpr int NI = R + 4;
 };
 
 // Block size for n envs: spread over all SMs first (a multiple of one warp), then grow up to kMaxBlock.
@@ -91,95 +80,20 @@ __device__ __forceinline__ const double *stage_trig_table() {
 __device__ __forceinline__ double *env_smem_base() { return rr_smem + kTrigRows * 4 + threadIdx.x; }
 __device__ __forceinline__ int env_smem_offset() { return kTrigRows * 4 + (int)threadIdx.x; }
 
-// HBM column -> (hot shared / cold local) fields.  Robot columns: cx,cy,l,r,t,b,rot,hx,hy,hrot.
-template <class L>
-__device__ __forceinline__ void load_env(typename L::E &e, double *cold, const Consts &k, const double *__restrict__ sf,
-                                         const int32_t *__restrict__ si, int64_t N, int64_t i) {
+// Bind e's hot fields to this thread's column of the shared-memory area and its cold fields to `cold`.
+template <class E>
+__device__ __forceinline__ void bind_env(E &e, double *cold) {
   e.base = env_smem_base();
   e.boff = env_smem_offset();
   e.cold = cold;
   e.stride = (int)blockDim.x;
-  e.memo_clear();
-  e.sq_watch = 0; e.rr_stuck = 0;
-  int f = 0;
-  e.hvalid = 0;
-  e.thrust = 0;
-  e.masks_dirty = true;
-  e.br_near = e.bb_near = e.rr_near = e.wall_near = e.moving = 0;
-#pragma unroll 1
-  for (int r = 0; r < L::R; r++) {
-#pragma unroll
-    for (int q = 0; q < 7; q++) e.rf(r, q) = sf[(f + q) * N + i];
-#pragma unroll
-    for (int q = 0; q < 3; q++) e.rc(r, q) = sf[(f + 7 + q) * N + i];
-    e.rc(r, 3) = rr_nan(); e.rc(r, 8) = rr_nan();  // heading-keyed caches start empty
-    f += L::kRobotF;
-    unpack_robot_word(e, r, si[r * N + i]);
-    robot_refresh_corners(e, k, r);
-  }
-#pragma unroll 1
-  for (int b = 0; b < L::B; b++) {
-#pragma unroll
-    for (int q = 0; q < L::kBallF; q++) e.bf(b, q) = sf[(f + q) * N + i];
-    f += L::kBallF;
-  }
-  e.ret_h = sf[(f + 0) * N + i]; e.ret_g = sf[(f + 1) * N + i];
-  f += 2;
-  if (k.observer == RR_OBS_ALLCOORDS_PRIOR) {
-#pragma unroll 1
-    for (int r = 0; r < L::R; r++, f += 3) {
-      e.rc(r, 13) = sf[(f + 0) * N + i]; e.rc(r, 14) = sf[(f + 1) * N + i]; e.rc(r, 15) = sf[(f + 2) * N + i];
-    }
-#pragma unroll 1
-    for (int b = 0; b < L::B; b++, f += 2) { e.bf(b, 8) = sf[(f + 0) * N + i]; e.bf(b, 9) = sf[(f + 1) * N + i]; }
-  }
-  e.step = si[(L::R + 0) * N + i];
-  e.episode = (unsigned)si[(L::R + 1) * N + i];
-  e.err = (unsigned)si[(L::R + 2) * N + i];
-  e.goal_clear();
-  if constexpr (L::E::kGoals) {  // goal bookkeeping: alive mask, scored masks, dwell counters [2][B] (extra int32 columns)
-#pragma unroll 1
-    for (int q = 0; q < L::E::kGoalDoubles; q++) e.gs(q) = (double)(unsigned)si[(L::R + 4 + q) * N + i];
-  }
 }
 
 template <class L>
-__device__ __forceinline__ void store_env(const typename L::E &e, const Consts &k, double *__restrict__ sf,
-                                          int32_t *__restrict__ si, int64_t N, int64_t i, int last_naughty) {
-  int f = 0;
-#pragma unroll 1
-  for (int r = 0; r < L::R; r++) {
-#pragma unroll
-    for (int q = 0; q < 7; q++) sf[(f + q) * N + i] = e.rf(r, q);
-#pragma unroll
-    for (int q = 0; q < 3; q++) sf[(f + 7 + q) * N + i] = e.rc(r, q);
-    f += L::kRobotF;
-    si[r * N + i] = pack_robot_word(e, r);
-  }
-#pragma unroll 1
-  for (int b = 0; b < L::B; b++) {
-#pragma unroll
-    for (int q = 0; q < L::kBallF; q++) sf[(f + q) * N + i] = e.bf(b, q);
-    f += L::kBallF;
-  }
-  sf[(f + 0) * N + i] = e.ret_h; sf[(f + 1) * N + i] = e.ret_g;
-  f += 2;
-  if (k.observer == RR_OBS_ALLCOORDS_PRIOR) {
-#pragma unroll 1
-    for (int r = 0; r < L::R; r++, f += 3) {
-      sf[(f + 0) * N + i] = e.rc(r, 13); sf[(f + 1) * N + i] = e.rc(r, 14); sf[(f + 2) * N + i] = e.rc(r, 15);
-    }
-#pragma unroll 1
-    for (int b = 0; b < L::B; b++, f += 2) { sf[(f + 0) * N + i] = e.bf(b, 8); sf[(f + 1) * N + i] = e.bf(b, 9); }
-  }
-  si[(L::R + 0) * N + i] = e.step;
-  si[(L::R + 1) * N + i] = (int32_t)e.episode;
-  si[(L::R + 2) * N + i] = (int32_t)e.err;
-  si[(L::R + 3) * N + i] = last_naughty;
-  if constexpr (L::E::kGoals) {
-#pragma unroll 1
-    for (int q = 0; q < L::E::kGoalDoubles; q++) si[(L::R + 4 + q) * N + i] = (int32_t)(unsigned)e.gs(q);
-  }
+__device__ __forceinline__ void load_env(typename L::E &e, double *cold, const Consts &k, const double *__restrict__ sf,
+                                         const int32_t *__restrict__ si, int64_t N, int64_t i) {
+  bind_env(e, cold);
+  load_columns(e, k, sf, si, N, i);
 }
 
 // Result rows of one warp: lane l holds `dim` values that belong at dst[l * dim .. l * dim + dim), so the warp's 32 rows
@@ -263,7 +177,7 @@ __global__ void __launch_bounds__(L::kMaxBlock, L::kStepBlocksPerSM) k_step(cons
   if (live) {
     load_env<L>(e, cold, k, a.sf, a.si, a.N, i);
   } else {
-    e.base = env_smem_base(); e.boff = env_smem_offset(); e.cold = cold; e.stride = (int)blockDim.x;
+    bind_env(e, cold);
     e.err = 0; e.step = 0; e.masks_dirty = false; e.sq_watch = 0; e.rr_stuck = 0;
   }
   const int dim = obs_dim_of<E>(k.observer);
@@ -376,7 +290,7 @@ __global__ void __launch_bounds__(L::kMaxBlock, L::kStepBlocksPerSM) k_step(cons
 #endif
   if (live) {
     st[RR_STAT_REPLAYS] = e.mm(kMReplays);
-    store_env<L>(e, k, a.sf, a.si, a.N, i, last_naughty);
+    store_columns(e, k, a.sf, a.si, a.N, i, last_naughty);
   }
   // episode statistics: warp-shuffle reduction, one atomic per warp and statistic
 #pragma unroll
@@ -395,14 +309,11 @@ __global__ void __launch_bounds__(L::kMaxBlock, 1) k_init(const __grid_constant_
   typename L::E e;
   double cold[L::E::kColdDoubles];
   e.trig = trig_tab;
-  e.base = env_smem_base();
-  e.boff = env_smem_offset();
-  e.cold = cold;
-  e.stride = (int)blockDim.x;
+  bind_env(e, cold);
   construct_env(e);
   reset_env(e, k, (uint64_t)(k.env_offset + i));
   record_start(e, start + i, N);  // _lst_starting_positions = _set_random_positions() (RR_EnvBase.py:112-113)
-  store_env<L>(e, k, sf, si, N, i, 0);
+  store_columns(e, k, sf, si, N, i, 0);
 }
 
 template <class L>
@@ -424,7 +335,7 @@ __global__ void __launch_bounds__(L::kMaxBlock, 1) k_reset_fixed(const __grid_co
   }
   e.episode += 1;
   reset_env_fixed(e, k, start + i, N);
-  store_env<L>(e, k, sf, si, N, i, 0);
+  store_columns(e, k, sf, si, N, i, 0);
 }
 
 template <class L>
@@ -440,7 +351,7 @@ __global__ void __launch_bounds__(L::kMaxBlock, 1) k_reset(const __grid_constant
   load_env<L>(e, cold, k, sf, si, N, i);
   e.episode += 1;
   reset_env(e, k, (uint64_t)(k.env_offset + i));
-  store_env<L>(e, k, sf, si, N, i, 0);
+  store_columns(e, k, sf, si, N, i, 0);
 }
 
 template <class L, typename OutT>
@@ -525,7 +436,7 @@ struct rr_sim {
   int64_t N;
   int device;
   int sms = 148;
-  int NH, NG, NP, NN, R, B, NF, NI;
+  Columns cols;                 // the layout of sf / si (rr_sim.cuh)
   double *sf = nullptr;
   int32_t *si = nullptr;
   double *start = nullptr;      // [3R + 2B][N] starting layout (_lst_starting_positions)
@@ -654,11 +565,6 @@ static cudaError_t opt_in_shared_memory() {
     else LAUNCH_ONE(LTrainGoals, s, st, KERNEL, __VA_ARGS__);                                               \
   } while (0)
 
-// columns of sf behind the base state: rectDblPriorStep poses, kept only for the observer that reports them
-static inline int prior_columns(const rr_sim *s) {
-  return s->cfg.observer == RR_OBS_ALLCOORDS_PRIOR ? 3 * s->R + 2 * s->B : 0;
-}
-
 int rr_check_config(const rr_config *cfg) {
   if (!cfg) return fail(RR_E_INVALID, "null argument");
   if (cfg->abi_version != RR_ABI_VERSION) return fail(RR_E_INVALID, "abi_version mismatch");
@@ -700,13 +606,11 @@ int rr_create(const rr_config *cfg, int64_t n_envs, int device, rr_sim **out) {
   cudaDeviceGetAttribute(&s->sms, cudaDevAttrMultiProcessorCount, device);
   if (s->sms <= 0) s->sms = 148;
   const bool game = cfg->preset == RR_PRESET_GAME;
-  s->NH = game ? 2 : 1; s->NG = game ? 2 : 0; s->NP = game ? 4 : 1; s->NN = game ? 4 : 0;
-  s->R = s->NH + s->NG; s->B = s->NP + s->NN;
-  s->NF = s->R * 10 + s->B * 8 + 2;
-  s->NI = s->R + 4 + (cfg->goal_scoring ? 2 + 2 * s->B : 0);
-  if (cudaMalloc(&s->start, sizeof(double) * (3 * s->R + 2 * s->B) * n_envs) != cudaSuccess ||
-      cudaMalloc(&s->sf, sizeof(double) * (s->NF + prior_columns(s)) * n_envs) != cudaSuccess ||
-      cudaMalloc(&s->si, sizeof(int32_t) * s->NI * n_envs) != cudaSuccess ||
+  s->cols = cfg->goal_scoring ? (game ? LGameGoals::E::kCols : LTrainGoals::E::kCols)
+                              : (game ? LGame::E::kCols : LTrain::E::kCols);
+  if (cudaMalloc(&s->start, sizeof(double) * (3 * s->cols.R + 2 * s->cols.B) * n_envs) != cudaSuccess ||
+      cudaMalloc(&s->sf, sizeof(double) * s->cols.nf(cfg->observer) * n_envs) != cudaSuccess ||
+      cudaMalloc(&s->si, sizeof(int32_t) * s->cols.ni() * n_envs) != cudaSuccess ||
       cudaMalloc(&s->own_stats, sizeof(double) * RR_NUM_STATS) != cudaSuccess) {
     cudaGetLastError();
     rr_destroy(s);
@@ -764,8 +668,8 @@ int rr_destroy(rr_sim *s) {
 }
 
 int rr_num_envs(const rr_sim *s, int64_t *n) { if (!s || !n) return fail(RR_E_INVALID, "null"); *n = s->N; return RR_OK; }
-int rr_num_robots(const rr_sim *s) { return s ? s->R : RR_E_INVALID; }
-int rr_num_balls(const rr_sim *s) { return s ? s->B : RR_E_INVALID; }
+int rr_num_robots(const rr_sim *s) { return s ? s->cols.R : RR_E_INVALID; }
+int rr_num_balls(const rr_sim *s) { return s ? s->cols.B : RR_E_INVALID; }
 int rr_max_steps(const rr_sim *s) { return s ? s->k.T : RR_E_INVALID; }
 int rr_obs_dim(const rr_sim *s) {
   if (!s) return RR_E_INVALID;
@@ -773,14 +677,14 @@ int rr_obs_dim(const rr_sim *s) {
     case RR_OBS_BASIC_LIDAR: return 5;
     case RR_OBS_LIDAR6_V2: return 11;
     case RR_OBS_LIDAR6_V1: return 11;
-    case RR_OBS_ALLCOORDS: return 3 * s->R + 2 * s->B;
-    case RR_OBS_ALLCOORDS_PRIOR: return 6 * s->R + 4 * s->B;
+    case RR_OBS_ALLCOORDS: return 3 * s->cols.R + 2 * s->cols.B;
+    case RR_OBS_ALLCOORDS_PRIOR: return 6 * s->cols.R + 4 * s->cols.B;
     default: return 0;
   }
 }
 int64_t rr_launch_count(const rr_sim *s) { return s ? s->launches : 0; }
 int64_t rr_state_bytes_per_env(const rr_sim *s) {
-  return s ? (int64_t)(s->NF + prior_columns(s)) * 8 + (int64_t)s->NI * 4 : 0;
+  return s ? s->cols.bytes_per_env(s->cfg.observer) : 0;
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -927,7 +831,7 @@ int rr_set_starting_positions(rr_sim *s, const double *rob3, const double *ball2
   ON_DEVICE(s->device);
   CK(cudaDeviceSynchronize());
   const int64_t N = s->N;
-  const int R = s->R, B = s->B;
+  const int R = s->cols.R, B = s->cols.B;
   std::vector<double> st((size_t)(3 * R + 2 * B) * N);
   for (int64_t i = 0; i < N; i++) {
     for (int q = 0; q < 3 * R; q++) st[(size_t)q * N + i] = rob3[i * 3 * R + q];
@@ -942,7 +846,7 @@ int rr_get_starting_positions(rr_sim *s, double *rob3, double *ball2) {
   ON_DEVICE(s->device);
   CK(cudaDeviceSynchronize());
   const int64_t N = s->N;
-  const int R = s->R, B = s->B;
+  const int R = s->cols.R, B = s->cols.B;
   std::vector<double> st((size_t)(3 * R + 2 * B) * N);
   CK(cudaMemcpy(st.data(), s->start, sizeof(double) * st.size(), cudaMemcpyDeviceToHost));
   for (int64_t i = 0; i < N; i++) {
@@ -980,8 +884,8 @@ int rr_observe_entity(rr_sim *s, int32_t robot, int32_t ball, const int32_t *bal
   if (ob == RR_OBS_ALLCOORDS || ob == RR_OBS_ALLCOORDS_PRIOR)
     return fail(RR_E_INVALID, "Robot-specific state output not supported.");  // RR_Observers.py:59-60
   if (ob == RR_OBS_NONE) return fail(RR_E_INVALID, "this env has no observer");
-  if (robot < 0 || robot >= s->R) return fail(RR_E_INVALID, "robot index out of range");
-  if (!ball_dev && ball >= s->B) return fail(RR_E_INVALID, "ball index out of range");
+  if (robot < 0 || robot >= s->cols.R) return fail(RR_E_INVALID, "robot index out of range");
+  if (!ball_dev && ball >= s->cols.B) return fail(RR_E_INVALID, "ball index out of range");
   if (misaligned(obs, out_size(s)) || misaligned(ball_dev, 4))
     return fail(RR_E_INVALID, "obs and ball_dev must be aligned to their element types");
   ON_DEVICE(s->device);
@@ -998,11 +902,11 @@ int rr_observe_entity(rr_sim *s, int32_t robot, int32_t ball, const int32_t *bal
 
 int rr_assign_balls(rr_sim *s, const int32_t *robots_host, int32_t n_robots, int32_t *assign_dev, void *stream) {
   if (!s || !robots_host || !assign_dev) return fail(RR_E_INVALID, "null argument");
-  if (n_robots < 1 || n_robots > s->R || n_robots > 8) return fail(RR_E_INVALID, "n_robots out of range");
+  if (n_robots < 1 || n_robots > s->cols.R || n_robots > 8) return fail(RR_E_INVALID, "n_robots out of range");
   RobotList rl{};
   rl.n = n_robots;
   for (int j = 0; j < n_robots; j++) {
-    if (robots_host[j] < 0 || robots_host[j] >= s->R) return fail(RR_E_INVALID, "robot index out of range");
+    if (robots_host[j] < 0 || robots_host[j] >= s->cols.R) return fail(RR_E_INVALID, "robot index out of range");
     rl.idx[j] = robots_host[j];
   }
   ON_DEVICE(s->device);
@@ -1018,10 +922,10 @@ static int check_actions(const rr_sim *s, int32_t n_actions, int32_t k_steps) {
   if (k_steps <= 0) return fail(RR_E_INVALID, "k_steps must be positive");
   if (n_actions < 0) return fail(RR_E_INVALID, "n_actions must be >= 0");
   // RR_EnvBase.py:621-622 / :270-271: more commands than robots (engines) raises
-  if (s->cfg.discrete && n_actions > s->R)
-    return fail(RR_E_INVALID, std::to_string(n_actions) + " commands but only " + std::to_string(s->R) + " robots.");
-  if (!s->cfg.discrete && (n_actions > 2 * s->R || (n_actions & 1)))
-    return fail(RR_E_INVALID, std::to_string(n_actions) + " commands but only " + std::to_string(2 * s->R) + " robot engines.");
+  if (s->cfg.discrete && n_actions > s->cols.R)
+    return fail(RR_E_INVALID, std::to_string(n_actions) + " commands but only " + std::to_string(s->cols.R) + " robots.");
+  if (!s->cfg.discrete && (n_actions > 2 * s->cols.R || (n_actions & 1)))
+    return fail(RR_E_INVALID, std::to_string(n_actions) + " commands but only " + std::to_string(2 * s->cols.R) + " robot engines.");
   return RR_OK;
 }
 
@@ -1165,7 +1069,7 @@ int rr_step_host(rr_sim *s, const void *actions, int32_t n_actions, int32_t k_st
     CK(cudaStreamCreateWithFlags(&s->copy_stream, cudaStreamNonBlocking));
     for (cudaEvent_t &e : s->chunk_done) CK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
   }
-  int chunks = s->host_chunks > 0 ? s->host_chunks : (s->R > 1 ? 1 : 4);
+  int chunks = s->host_chunks > 0 ? s->host_chunks : (s->cols.R > 1 ? 1 : 4);
   if (chunks > 4) chunks = 4;
   if (chunks < 1 || k_steps < chunks) chunks = 1;
   const size_t act_row = (size_t)s->N * n_actions * (s->cfg.discrete ? 1 : 4);
@@ -1245,7 +1149,7 @@ int rr_set_state(rr_sim *s, const double *rob, const double *rhist, const int32_
                  const int32_t *step) {
   if (!s || !rob || !rhist || !rflag || !ball || !step) return fail(RR_E_INVALID, "null argument");
   const int64_t N = s->N;
-  const int R = s->R, B = s->B;
+  const int R = s->cols.R, B = s->cols.B;
   for (int64_t q = 0; q < N * R; q++) {  // what the packed si column can hold (Env::thrust: 4 bits per thrust)
     const int32_t *g = rflag + 3 * q;
     if (g[0] < -8 || g[0] > 7 || g[1] < -8 || g[1] > 7 || (g[2] != 0 && g[2] != 1))
@@ -1254,52 +1158,12 @@ int rr_set_state(rr_sim *s, const double *rob, const double *rhist, const int32_
   }
   ON_DEVICE(s->device);
   CK(cudaDeviceSynchronize());
-  const int NFP = s->NF + prior_columns(s);
-  std::vector<double> sf((size_t)NFP * N);
-  std::vector<int32_t> si((size_t)s->NI * N);
+  std::vector<double> sf((size_t)s->cols.nf(s->cfg.observer) * N);
+  std::vector<int32_t> si((size_t)s->cols.ni() * N);
   CK(cudaMemcpy(si.data(), s->si, sizeof(int32_t) * si.size(), cudaMemcpyDeviceToHost));  // keep episode counters
-  for (int64_t i = 0; i < N; i++) {
-    int f = 0;
-    for (int r = 0; r < R; r++) {
-      const double *p = rob + (i * R + r) * 7;
-      for (int q = 0; q < 7; q++) sf[(size_t)(f + q) * N + i] = p[q];
-      const double *h = rhist + (i * R + r) * 3;
-      for (int q = 0; q < 3; q++) sf[(size_t)(f + 7 + q) * N + i] = h[q];
-      f += 10;
-      const int32_t *g = rflag + (i * R + r) * 3;
-      si[(size_t)r * N + i] = (g[0] & 0xff) | ((g[1] & 0xff) << 8) | (g[2] << 16);
-    }
-    for (int b = 0; b < B; b++) {
-      const double *p = ball + (i * B + b) * 8;
-      for (int q = 0; q < 8; q++) sf[(size_t)(f + q) * N + i] = p[q];
-      f += 8;
-    }
-    sf[(size_t)(f + 0) * N + i] = 0.0; sf[(size_t)(f + 1) * N + i] = 0.0;
-    f += 2;
-    if (prior_columns(s)) {
-      // rectDblPriorStep of the injected state = rectDbl.copy() of the injected pose, as every on_reset / on_step_begin
-      // leaves it (RR_Robot.py:83,117; RR_Ball.py:56,61,76; snapshot_prior_step in rr_sim.cuh): the observation of an
-      // injected state is then the same as the reference's ref_harness.inject(), which copies the rects too
-      for (int r = 0; r < R; r++, f += 3) {
-        const double *p = rob + (i * R + r) * 7;
-        sf[(size_t)(f + 0) * N + i] = norm_rot(p[6]);
-        sf[(size_t)(f + 1) * N + i] = 10.0 + (p[0] - 10.0);
-        sf[(size_t)(f + 2) * N + i] = 20.0 + (p[1] - 20.0);
-      }
-      for (int b = 0; b < B; b++, f += 2) {
-        const double *p = ball + (i * B + b) * 8;
-        sf[(size_t)(f + 0) * N + i] = 7.0 + (p[0] - 7.0);
-        sf[(size_t)(f + 1) * N + i] = 7.0 + (p[1] - 7.0);
-      }
-    }
-    si[(size_t)(R + 0) * N + i] = step[i];
-    si[(size_t)(R + 2) * N + i] = 0;
-    si[(size_t)(R + 3) * N + i] = 0;
-    if (s->cfg.goal_scoring) {  // as after a reset: every ball alive, nothing tracked or scored
-      si[(size_t)(R + 4) * N + i] = (1 << B) - 1;
-      for (int q = 1; q < 2 + 2 * B; q++) si[(size_t)(R + 4 + q) * N + i] = 0;
-    }
-  }
+  for (int64_t i = 0; i < N; i++)
+    state_to_columns(s->cols, s->cfg.observer, sf.data(), si.data(), N, i, rob + i * R * 7, rhist + i * R * 3,
+                     rflag + i * R * 3, ball + i * B * 8, step[i]);
   CK(cudaMemcpy(s->sf, sf.data(), sizeof(double) * sf.size(), cudaMemcpyHostToDevice));
   CK(cudaMemcpy(s->si, si.data(), sizeof(int32_t) * si.size(), cudaMemcpyHostToDevice));
   return RR_OK;
@@ -1310,30 +1174,14 @@ int rr_get_state(rr_sim *s, double *rob, double *rhist, int32_t *rflag, double *
   ON_DEVICE(s->device);
   CK(cudaDeviceSynchronize());
   const int64_t N = s->N;
-  const int R = s->R, B = s->B;
-  std::vector<double> sf((size_t)s->NF * N);
-  std::vector<int32_t> si((size_t)s->NI * N);
+  const int R = s->cols.R, B = s->cols.B;
+  std::vector<double> sf((size_t)s->cols.nf_base() * N);
+  std::vector<int32_t> si((size_t)s->cols.ni() * N);
   CK(cudaMemcpy(sf.data(), s->sf, sizeof(double) * sf.size(), cudaMemcpyDeviceToHost));
   CK(cudaMemcpy(si.data(), s->si, sizeof(int32_t) * si.size(), cudaMemcpyDeviceToHost));
-  for (int64_t i = 0; i < N; i++) {
-    int f = 0;
-    for (int r = 0; r < R; r++) {
-      double *p = rob + (i * R + r) * 7;
-      for (int q = 0; q < 7; q++) p[q] = sf[(size_t)(f + q) * N + i];
-      int32_t pk = si[(size_t)r * N + i];
-      int32_t *g = rflag + (i * R + r) * 3;
-      g[0] = (int8_t)(pk & 0xff); g[1] = (int8_t)((pk >> 8) & 0xff); g[2] = (pk >> 16) & 1;
-      double *h = rhist + (i * R + r) * 3;
-      for (int q = 0; q < 3; q++) h[q] = g[2] ? sf[(size_t)(f + 7 + q) * N + i] : 0.0;
-      f += 10;
-    }
-    for (int b = 0; b < B; b++) {
-      double *p = ball + (i * B + b) * 8;
-      for (int q = 0; q < 8; q++) p[q] = sf[(size_t)(f + q) * N + i];
-      f += 8;
-    }
-    step[i] = si[(size_t)(R + 0) * N + i];
-  }
+  for (int64_t i = 0; i < N; i++)
+    state_from_columns(s->cols, sf.data(), si.data(), N, i, rob + i * R * 7, rhist + i * R * 3, rflag + i * R * 3,
+                       ball + i * B * 8, step + i);
   return RR_OK;
 }
 
@@ -1343,9 +1191,9 @@ int rr_goal_state(rr_sim *s, int32_t *alive_host, int32_t *score_host, int32_t *
   ON_DEVICE(s->device);
   CK(cudaDeviceSynchronize());
   const int64_t N = s->N;
-  const int R = s->R, B = s->B, G = 2 + 2 * B;
-  std::vector<int32_t> g((size_t)G * N);
-  CK(cudaMemcpy(g.data(), s->si + (size_t)(R + 4) * N, sizeof(int32_t) * g.size(), cudaMemcpyDeviceToHost));
+  const int B = s->cols.B;
+  std::vector<int32_t> g((size_t)s->cols.G * N);
+  CK(cudaMemcpy(g.data(), s->si + (size_t)s->cols.goal(0) * N, sizeof(int32_t) * g.size(), cudaMemcpyDeviceToHost));
   const uint32_t bm = (1u << B) - 1u;
   for (int64_t i = 0; i < N; i++) {
     const uint32_t alive = (uint32_t)g[(size_t)0 * N + i], sc = (uint32_t)g[(size_t)1 * N + i];
@@ -1367,7 +1215,7 @@ int rr_error_mask(rr_sim *s, uint32_t *err_host, int32_t clear) {
   if (!s || !err_host) return fail(RR_E_INVALID, "null argument");
   ON_DEVICE(s->device);
   CK(cudaDeviceSynchronize());
-  int32_t *p = s->si + (size_t)(s->R + 2) * s->N;
+  int32_t *p = s->si + (size_t)s->cols.err() * s->N;
   CK(cudaMemcpy(err_host, p, sizeof(uint32_t) * s->N, cudaMemcpyDeviceToHost));
   if (clear) CK(cudaMemset(p, 0, sizeof(uint32_t) * s->N));
   return RR_OK;
@@ -1377,7 +1225,7 @@ int rr_last_naughty(rr_sim *s, int32_t *count_host) {
   if (!s || !count_host) return fail(RR_E_INVALID, "null argument");
   ON_DEVICE(s->device);
   CK(cudaDeviceSynchronize());
-  CK(cudaMemcpy(count_host, s->si + (size_t)(s->R + 3) * s->N, sizeof(int32_t) * s->N, cudaMemcpyDeviceToHost));
+  CK(cudaMemcpy(count_host, s->si + (size_t)s->cols.naughty() * s->N, sizeof(int32_t) * s->N, cudaMemcpyDeviceToHost));
   return RR_OK;
 }
 

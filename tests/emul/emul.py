@@ -61,7 +61,7 @@ def lib():
         L.emul_step_k.argtypes = [C.POINTER(Config), vp, vp, vp, vp, vp, vp, C.c_int, C.c_int, vp, vp]
         L.emul_step_k.restype = C.c_uint
         i64 = C.c_int64
-        L.emul_cols_dims.argtypes = [C.POINTER(Config), vp, vp]
+        L.emul_cols_dims.argtypes = [C.POINTER(Config), vp]
         L.emul_cols_dims.restype = None
         L.emul_cols_set_state.argtypes = [C.POINTER(Config), vp, vp, i64, i64, vp, vp, vp, vp, C.c_int32]
         L.emul_cols_set_state.restype = None
@@ -155,14 +155,15 @@ class EmulEnv:
 
 
 class EmulBatch:
-    """M envs whose complete state persists between calls in the HBM layout of rr_b200.cu (sf [NF][M], si [NI][M]):
+    """M envs whose complete state persists between calls in the kernels' HBM layout (rr::Columns in rr_sim.cuh):
     launch() does what one k_step launch does, with the bookkeeping and auto-reset of the kernel source."""
 
     def __init__(self, cfg, M, R, B, obs_dim):
         self.cfg, self.M, self.R, self.B, self.obs_dim = cfg, M, R, B, obs_dim
-        nf = np.zeros(1, np.int32); ni = np.zeros(1, np.int32)
-        lib().emul_cols_dims(C.byref(cfg), _p(nf), _p(ni))
-        self.sf = np.zeros((int(nf[0]), M)); self.si = np.zeros((int(ni[0]), M), np.int32)
+        dims = np.zeros(5, np.int32)
+        lib().emul_cols_dims(C.byref(cfg), _p(dims))
+        nf, ni, self._episode_row, self._err_row, self._naughty_row = (int(d) for d in dims)
+        self.sf = np.zeros((nf, M)); self.si = np.zeros((ni, M), np.int32)
         self.reset(create=True)
 
     def reset(self, mask=None, create=False):
@@ -188,17 +189,17 @@ class EmulBatch:
 
     @property
     def episode(self):
-        return self.si[self.R + 1].copy()
+        return self.si[self._episode_row].copy()
 
     def error_mask(self, clear=False):
         """rr_error_mask."""
-        m = self.si[self.R + 2].astype(np.uint32)
+        m = self.si[self._err_row].astype(np.uint32)
         if clear:
-            self.si[self.R + 2] = 0
+            self.si[self._err_row] = 0
         return m
 
     def last_naughty(self):
-        return self.si[self.R + 3].copy()
+        return self.si[self._naughty_row].copy()
 
     def launch(self, actions, observe=False):
         """One launch of K steps; actions [K, M, A].  Returns dict(rew [K, M, 2], done, err (the row's error bits),

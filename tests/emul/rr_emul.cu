@@ -181,73 +181,14 @@ static unsigned reset_t(const Consts &k, double *rob, double *rhist, int32_t *rf
 }
 
 // ---- k_step launches on the host ---------------------------------------------------------------------------------------
-// The persistent state of M envs in the HBM layout of rr_b200.cu (sf [NF][M] doubles, si [NI][M] int32: see the top of
-// that file); col_load / col_store mirror its load_env / store_env, emul_launch one k_step launch over all M envs.
-template <class E>
-struct Cols {
-  static constexpr int R = E::R, B = E::B;
-  static constexpr int NF_BASE = R * 10 + B * 8 + 2;
-  static constexpr int NF = NF_BASE + 3 * R + 2 * B;
-  static constexpr int NI = R + 4 + E::kGoalDoubles;
-};
-
+// The persistent state of M envs in the kernels' HBM layout (rr::Columns in rr_sim.cuh), moved in and out of an Env by
+// the kernels' own load_columns / store_columns; emul_launch is one k_step launch over all M envs.
 template <class E>
 static void col_load(E &e, const Consts &k, const double *sf, const int32_t *si, int64_t N, int64_t i) {
-  // a launch starts from nothing but the stored columns: every field load_env does not set holds NaN here
+  // a launch starts from nothing but the stored columns: every field load_columns does not set holds NaN here
   for (int q = 0; q < E::kDoubles; q++) e.base[q] = HUGE_VAL - HUGE_VAL;
   for (int q = 0; q < E::kColdDoubles; q++) e.cold[q] = HUGE_VAL - HUGE_VAL;
-  e.memo_clear();
-  e.sq_watch = 0; e.rr_stuck = 0;
-  e.hvalid = 0; e.thrust = 0; e.masks_dirty = true;
-  e.br_near = e.bb_near = e.rr_near = e.wall_near = e.moving = 0;
-  int f = 0;
-  for (int r = 0; r < E::R; r++, f += 10) {
-    for (int q = 0; q < 7; q++) e.rf(r, q) = sf[(f + q) * N + i];
-    for (int q = 0; q < 3; q++) e.rc(r, q) = sf[(f + 7 + q) * N + i];
-    e.rc(r, 3) = rr_nan(); e.rc(r, 8) = rr_nan();
-    unpack_robot_word(e, r, si[r * N + i]);
-    robot_refresh_corners(e, k, r);
-  }
-  for (int b = 0; b < E::B; b++, f += 8)
-    for (int q = 0; q < 8; q++) e.bf(b, q) = sf[(f + q) * N + i];
-  e.ret_h = sf[(f + 0) * N + i]; e.ret_g = sf[(f + 1) * N + i];
-  f += 2;
-  if (k.observer == RR_OBS_ALLCOORDS_PRIOR) {
-    for (int r = 0; r < E::R; r++, f += 3) {
-      e.rc(r, 13) = sf[(f + 0) * N + i]; e.rc(r, 14) = sf[(f + 1) * N + i]; e.rc(r, 15) = sf[(f + 2) * N + i];
-    }
-    for (int b = 0; b < E::B; b++, f += 2) { e.bf(b, 8) = sf[(f + 0) * N + i]; e.bf(b, 9) = sf[(f + 1) * N + i]; }
-  }
-  e.step = si[(E::R + 0) * N + i];
-  e.episode = (unsigned)si[(E::R + 1) * N + i];
-  e.err = (unsigned)si[(E::R + 2) * N + i];
-  e.goal_clear();
-  for (int q = 0; q < E::kGoalDoubles; q++) e.gs(q) = (double)(unsigned)si[(E::R + 4 + q) * N + i];
-}
-
-template <class E>
-static void col_store(const E &e, const Consts &k, double *sf, int32_t *si, int64_t N, int64_t i, int last_naughty) {
-  int f = 0;
-  for (int r = 0; r < E::R; r++, f += 10) {
-    for (int q = 0; q < 7; q++) sf[(f + q) * N + i] = e.rf(r, q);
-    for (int q = 0; q < 3; q++) sf[(f + 7 + q) * N + i] = e.rc(r, q);
-    si[r * N + i] = pack_robot_word(e, r);
-  }
-  for (int b = 0; b < E::B; b++, f += 8)
-    for (int q = 0; q < 8; q++) sf[(f + q) * N + i] = e.bf(b, q);
-  sf[(f + 0) * N + i] = e.ret_h; sf[(f + 1) * N + i] = e.ret_g;
-  f += 2;
-  if (k.observer == RR_OBS_ALLCOORDS_PRIOR) {
-    for (int r = 0; r < E::R; r++, f += 3) {
-      sf[(f + 0) * N + i] = e.rc(r, 13); sf[(f + 1) * N + i] = e.rc(r, 14); sf[(f + 2) * N + i] = e.rc(r, 15);
-    }
-    for (int b = 0; b < E::B; b++, f += 2) { sf[(f + 0) * N + i] = e.bf(b, 8); sf[(f + 1) * N + i] = e.bf(b, 9); }
-  }
-  si[(E::R + 0) * N + i] = e.step;
-  si[(E::R + 1) * N + i] = (int32_t)e.episode;
-  si[(E::R + 2) * N + i] = (int32_t)e.err;
-  si[(E::R + 3) * N + i] = last_naughty;
-  for (int q = 0; q < E::kGoalDoubles; q++) si[(E::R + 4 + q) * N + i] = (int32_t)(unsigned)e.gs(q);
+  load_columns(e, k, sf, si, N, i);
 }
 
 // One k_step launch: K steps of every env, actions [K][M][A] as doubles (see decode_actions).  Rows: rew [K][M][2],
@@ -281,7 +222,7 @@ static void launch_t(const Consts &k, double *sf, int32_t *si, int64_t M, const 
       if (obs_g) observe(e, k, -1, obs_g + row * dim, oerr);
     }
     st[RR_STAT_REPLAYS] = e.mm(kMReplays);
-    col_store(e, k, sf, si, M, i, last_naughty);
+    store_columns(e, k, sf, si, M, i, last_naughty);
     for (int q = 0; q < RR_NUM_STATS; q++) stats[i * RR_NUM_STATS + q] = st[q];
   }
 }
@@ -300,60 +241,8 @@ static void cols_reset_t(const Consts &k, double *sf, int32_t *si, int64_t M, co
       e.episode += 1;
     }
     reset_env(e, k, (uint64_t)(k.env_offset + i));
-    col_store(e, k, sf, si, M, i, 0);
+    store_columns(e, k, sf, si, M, i, 0);
   }
-}
-
-// rr_set_state / rr_get_state for env i of the columns (one env's arrays as in include/rr_b200.h)
-template <class E>
-static void cols_set_state(const rr_config &c, double *sf, int32_t *si, int64_t N, int64_t i, const double *rob,
-                           const double *rhist, const int32_t *rflag, const double *ball, int32_t step) {
-  constexpr int R = E::R, B = E::B;
-  int f = 0;
-  for (int r = 0; r < R; r++, f += 10) {
-    for (int q = 0; q < 7; q++) sf[(f + q) * N + i] = rob[r * 7 + q];
-    for (int q = 0; q < 3; q++) sf[(f + 7 + q) * N + i] = rhist[r * 3 + q];
-    const int32_t *g = rflag + r * 3;
-    si[r * N + i] = (g[0] & 0xff) | ((g[1] & 0xff) << 8) | (g[2] << 16);
-  }
-  for (int b = 0; b < B; b++, f += 8)
-    for (int q = 0; q < 8; q++) sf[(f + q) * N + i] = ball[b * 8 + q];
-  sf[(f + 0) * N + i] = 0.0; sf[(f + 1) * N + i] = 0.0;
-  f += 2;
-  if (c.observer == RR_OBS_ALLCOORDS_PRIOR) {
-    for (int r = 0; r < R; r++, f += 3) {
-      sf[(f + 0) * N + i] = norm_rot(rob[r * 7 + 6]);
-      sf[(f + 1) * N + i] = 10.0 + (rob[r * 7 + 0] - 10.0);
-      sf[(f + 2) * N + i] = 20.0 + (rob[r * 7 + 1] - 20.0);
-    }
-    for (int b = 0; b < B; b++, f += 2) {
-      sf[(f + 0) * N + i] = 7.0 + (ball[b * 8 + 0] - 7.0);
-      sf[(f + 1) * N + i] = 7.0 + (ball[b * 8 + 1] - 7.0);
-    }
-  }
-  si[(R + 0) * N + i] = step;
-  si[(R + 2) * N + i] = 0;
-  si[(R + 3) * N + i] = 0;
-  if (E::kGoals) {
-    si[(R + 4) * N + i] = (1 << B) - 1;
-    for (int q = 1; q < 2 + 2 * B; q++) si[(R + 4 + q) * N + i] = 0;
-  }
-}
-
-template <class E>
-static void cols_get_state(const double *sf, const int32_t *si, int64_t N, int64_t i, double *rob, double *rhist,
-                           int32_t *rflag, double *ball, int32_t *step) {
-  int f = 0;
-  for (int r = 0; r < E::R; r++, f += 10) {
-    for (int q = 0; q < 7; q++) rob[r * 7 + q] = sf[(f + q) * N + i];
-    const int32_t pk = si[r * N + i];
-    int32_t *g = rflag + r * 3;
-    g[0] = (int8_t)(pk & 0xff); g[1] = (int8_t)((pk >> 8) & 0xff); g[2] = (pk >> 16) & 1;
-    for (int q = 0; q < 3; q++) rhist[r * 3 + q] = g[2] ? sf[(f + 7 + q) * N + i] : 0.0;
-  }
-  for (int b = 0; b < E::B; b++, f += 8)
-    for (int q = 0; q < 8; q++) ball[b * 8 + q] = sf[(f + q) * N + i];
-  *step = si[E::R * N + i];
 }
 
 // the Env type of a configuration: GAME 2 + 2 robots, 4 + 4 balls; TRAIN 1 robot, 1 ball; goal scoring compiled in or not
@@ -363,22 +252,8 @@ static void cols_get_state(const double *sf, const int32_t *si, int64_t N, int64
                        : ((cfg)->preset == RR_PRESET_GAME ? F<2, 2, 4, 4>(__VA_ARGS__) : F<1, 0, 1, 0>(__VA_ARGS__)))
 
 template <int NH, int NG, int NP, int NN, bool G = false>
-static int cols_dims_t(int32_t *nf, int32_t *ni) {
-  using C = Cols<Env<NH, NG, NP, NN, G>>;
-  *nf = C::NF; *ni = C::NI;
-  return 0;
-}
-template <int NH, int NG, int NP, int NN, bool G = false>
-static int cols_set_state_t(const rr_config *c, double *sf, int32_t *si, int64_t M, int64_t i, const double *rob,
-                            const double *rhist, const int32_t *rflag, const double *ball, int32_t step) {
-  cols_set_state<Env<NH, NG, NP, NN, G>>(*c, sf, si, M, i, rob, rhist, rflag, ball, step);
-  return 0;
-}
-template <int NH, int NG, int NP, int NN, bool G = false>
-static int cols_get_state_t(const double *sf, const int32_t *si, int64_t M, int64_t i, double *rob, double *rhist,
-                            int32_t *rflag, double *ball, int32_t *step) {
-  cols_get_state<Env<NH, NG, NP, NN, G>>(sf, si, M, i, rob, rhist, rflag, ball, step);
-  return 0;
+static Columns columns_t() {
+  return Env<NH, NG, NP, NN, G>::kCols;
 }
 template <int NH, int NG, int NP, int NN, bool G = false>
 static int launch_dispatch_t(const Consts &k, double *sf, int32_t *si, int64_t M, const double *actions, int A, int K,
@@ -395,16 +270,21 @@ static int reset_dispatch_t(const Consts &k, double *sf, int32_t *si, int64_t M,
 
 extern "C" {
 
-void emul_cols_dims(const rr_config *cfg, int32_t *nf, int32_t *ni) { EMUL_DISPATCH(cfg, cols_dims_t, nf, ni); }
+// dims = {sf columns, si columns, si column of the episode, of the error mask, of the last naughty count}
+void emul_cols_dims(const rr_config *cfg, int32_t *dims) {
+  const Columns C = EMUL_DISPATCH(cfg, columns_t);
+  const int32_t d[] = {C.nf(cfg->observer), C.ni(), C.episode(), C.err(), C.naughty()};
+  std::memcpy(dims, d, sizeof d);
+}
 
 void emul_cols_set_state(const rr_config *cfg, double *sf, int32_t *si, int64_t M, int64_t i, const double *rob,
                          const double *rhist, const int32_t *rflag, const double *ball, int32_t step) {
-  EMUL_DISPATCH(cfg, cols_set_state_t, cfg, sf, si, M, i, rob, rhist, rflag, ball, step);
+  state_to_columns(EMUL_DISPATCH(cfg, columns_t), cfg->observer, sf, si, M, i, rob, rhist, rflag, ball, step);
 }
 
 void emul_cols_get_state(const rr_config *cfg, const double *sf, const int32_t *si, int64_t M, int64_t i, double *rob,
                          double *rhist, int32_t *rflag, double *ball, int32_t *step) {
-  EMUL_DISPATCH(cfg, cols_get_state_t, sf, si, M, i, rob, rhist, rflag, ball, step);
+  state_from_columns(EMUL_DISPATCH(cfg, columns_t), sf, si, M, i, rob, rhist, rflag, ball, step);
 }
 
 void emul_cols_reset(const rr_config *cfg, double *sf, int32_t *si, int64_t M, const uint8_t *mask, int create) {

@@ -41,7 +41,7 @@ static int launch_info_t(const Consts &k, double *sf, int32_t *si, int64_t M, co
       if (obs_g) observe(e, k, -1, obs_g + row * dim, oerr);
     }
     st[RR_STAT_REPLAYS] = e.mm(kMReplays);
-    col_store(e, k, sf, si, M, i, last_naughty);
+    store_columns(e, k, sf, si, M, i, last_naughty);
     for (int q = 0; q < RR_NUM_STATS; q++) stats[i * RR_NUM_STATS + q] = st[q];
   }
   return 0;

@@ -605,7 +605,7 @@ def test_gpu_squeeze_memo_replay_is_exact(oracle, preset, fused):
         env.set_state(pool)
         if fused:
             out = [x.clone() for x in env.step_k(a, K)]
-        else:   # one launch per env-step: the memo record travels from launch to launch through HBM (load_env / store_env)
+        else:   # one launch per env-step: the memo record travels from launch to launch through HBM (load_columns / store_columns)
             rows = [[x.clone() for x in env.step_k(a[t:t + 1], 1)] for t in range(K)]
             out = [torch.cat([r[j] for r in rows]) for j in range(4)]
         torch.cuda.synchronize()
