@@ -287,6 +287,37 @@ int rr_set_state(rr_sim *s, const double *rob, const double *rhist, const int32_
                  const double *ball, const int32_t *step);
 int rr_get_state(rr_sim *s, double *rob, double *rhist, int32_t *rflag, double *ball, int32_t *step);
 
+/* Saved env states on the device: copy.deepcopy(env) of the reference, batched, without a host round trip (search and
+ * lookahead from a common root, "reset to an archived state" curricula, checkpoints of envs mid-episode, replaying an env
+ * that raised).  A saved env is one row of S = rr_snapshot_bytes_per_env(s) bytes (rr_sim.cuh RowLayout): every per-env
+ * column of the state (robots with their thrusts, history-valid bits and episode-counted bit, balls, episode returns,
+ * the AllCoords_WithPrior prior-step poses, step and episode counters, sticky error mask, last naughty count, goal
+ * words), the starting layout, then zero padding to a multiple of 16 bytes, so two saves of one state are byte-equal.
+ *   GAME  1104 (goal_scoring 1184, RR_OBS_ALLCOORDS_PRIOR 1328, both 1408)
+ *   TRAIN  224 (goal_scoring  240, RR_OBS_ALLCOORDS_PRIOR  272, both  288)
+ * The eight widths differ, so the width identifies the layout.  A row holds neither the statistics nor the pipeline and
+ * flush settings nor anything of rr_config.
+ * rr_save_states: for each j < m, row j of rows_dev (m rows of S bytes, 16-byte aligned) receives env env_dev[j]
+ *   (env_dev NULL: env j, and m <= N); duplicates are allowed; an index outside [0, N) leaves its row unwritten.
+ * rr_load_states: every env i with 0 <= slot_dev[i] < m receives row slot_dev[i]; a negative index (or one >= m) leaves
+ *   env i untouched (slot_dev NULL: env i receives row i, and m == N).  A gather: no two rows can write one env.
+ * Both are asynchronous and ordered on `stream` like rr_reset: they join the sub-batch pipeline into `stream` first (a
+ * save after rr_step sees the stepped state, the next rr_step sees a load), and each adds one launch to rr_launch_count.
+ * RR_E_INVALID, nothing launched: a NULL handle or rows pointer, m < 1, rows_dev not 16-byte aligned, an index pointer
+ * not 8-byte aligned, or m against the rule of a NULL index pointer.
+ * After a load every entry point reports for env i what it reported for the saved env at save time (rr_get_state,
+ * rr_observe, rr_observe_entity, rr_assign_balls, rr_goal_state, rr_error_mask, rr_last_naughty,
+ * rr_get_starting_positions), and stepping env i gives the saved env's rows bit for bit until a random reset, which
+ * draws with the DESTINATION's global env index and the row's episode counter: a row loaded back into the env it came
+ * from (same seed and env_offset) repeats even its resets, a clone in another env diverges from its first random reset
+ * on.  A row can be loaded into any handle of the same width (another handle, another process through host memory) and
+ * continues the same physical state under that handle's reward and observer configuration.  The statistics are not
+ * touched; the episode-counted bit travels with the row, so an episode already counted is not counted again and an
+ * uncounted one is counted each time a loaded copy of it finishes. */
+int64_t rr_snapshot_bytes_per_env(const rr_sim *s);
+int rr_save_states(rr_sim *s, const int64_t *env_dev, int64_t m, void *rows_dev, void *stream);
+int rr_load_states(rr_sim *s, const void *rows_dev, int64_t m, const int64_t *slot_dev, void *stream);
+
 /* Goal bookkeeping (goal_scoring = 1) to HOST; any pointer may be NULL.  alive[N]: bit b = ball b still in play;
  * score[N][2]: Goal.get_score() of the happy and the grumpy goal (RR_Goal.py:87-88); destroyed[N]: bit 0 happy goal,
  * bit 1 grumpy goal (Goal.is_destroyed, :90-91); dwell[N][2][B]: steps ball b has stayed inside that goal's triangle

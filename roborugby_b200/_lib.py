@@ -74,6 +74,9 @@ SIGNATURES = {
     "rr_step_host_end": (C.c_int, [_vp, _i32]),
     "rr_set_state": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp]),
     "rr_get_state": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp]),
+    "rr_snapshot_bytes_per_env": (_i64, [_vp]),
+    "rr_save_states": (C.c_int, [_vp, _vp, _i64, _vp, _vp]),
+    "rr_load_states": (C.c_int, [_vp, _vp, _i64, _vp, _vp]),
     "rr_goal_state": (C.c_int, [_vp, _vp, _vp, _vp, _vp]),
     "rr_error_mask": (C.c_int, [_vp, _vp, _i32]),
     "rr_last_naughty": (C.c_int, [_vp, _vp]),

@@ -423,6 +423,90 @@ __global__ void __launch_bounds__(L::kMaxBlock, 1) k_assign_balls(const __grid_c
   for (int j = 0; j < robots.n; j++) assign[i * robots.n + j] = out[j];
 }
 
+// Saved env rows (rr_save_states / rr_load_states; the layout is RowLayout in rr_sim.cuh).  A block moves a tile of 32 rows
+// through shared memory: the column side is accessed with lane = env, so that every load or store instruction touches one
+// column of 32 envs (coalesced when the envs are consecutive), and the row side with 128-bit accesses.  In shared memory a
+// row takes an odd number of 16-byte chunks, so that the 128-bit accesses of 32 lanes to chunk q of 32 rows hit distinct
+// banks.  Pure data movement: one kernel per direction serves every preset and observer.
+constexpr int kRowTile = 32, kRowThreads = 256, kRowWarps = kRowThreads / 32;
+RR_HD constexpr int row_tile_chunks(const RowLayout &L) { return (L.bytes() / 16) | 1; }
+constexpr size_t row_tile_bytes(const RowLayout &L) { return (size_t)kRowTile * row_tile_chunks(L) * 16; }
+constexpr int kRowBatch = 4;  // chunks a lane has in flight in the column-side loop
+
+__global__ void __launch_bounds__(kRowThreads) k_save_rows(const RowLayout L, const uint64_t *__restrict__ sf,
+                                                           const uint64_t *__restrict__ start,
+                                                           const uint32_t *__restrict__ si, int64_t N,
+                                                           const int64_t *__restrict__ env, int64_t m,
+                                                           uint4 *__restrict__ rows) {
+  extern __shared__ uint4 tile[];
+  __shared__ int64_t src[kRowTile];
+  const int Q = L.bytes() / 16, QS = row_tile_chunks(L);
+  const int64_t j0 = (int64_t)blockIdx.x * kRowTile;
+  const int nrows = m - j0 < kRowTile ? (int)(m - j0) : kRowTile;
+  if (threadIdx.x < kRowTile) src[threadIdx.x] = (int)threadIdx.x < nrows ? save_source(env, j0 + threadIdx.x, N) : -1;
+  __syncthreads();
+  // gather: lane = row of the tile, warp w takes chunks w, w + 8, ...
+  const int j = threadIdx.x & 31, w = threadIdx.x >> 5;
+  const int64_t e = src[j];
+  if (e >= 0) {
+#pragma unroll 1
+    for (int q0 = w; q0 < Q; q0 += kRowWarps * kRowBatch) {
+      uint64_t v[2 * kRowBatch];
+#pragma unroll
+      for (int t = 0; t < kRowBatch; t++) {
+        const int q = q0 + t * kRowWarps;
+        if (q < Q) { v[2 * t] = row_unit_get(L, sf, start, si, N, e, 2 * q); v[2 * t + 1] = row_unit_get(L, sf, start, si, N, e, 2 * q + 1); }
+      }
+#pragma unroll
+      for (int t = 0; t < kRowBatch; t++) {
+        const int q = q0 + t * kRowWarps;
+        if (q < Q)
+          tile[j * QS + q] = make_uint4((unsigned)v[2 * t], (unsigned)(v[2 * t] >> 32), (unsigned)v[2 * t + 1],
+                                        (unsigned)(v[2 * t + 1] >> 32));
+      }
+    }
+  }
+  __syncthreads();
+  // the tile's rows are one contiguous range of the output: 128-bit stores (rows of skipped indices are not written)
+  uint4 *dst = rows + j0 * Q;
+#pragma unroll 4
+  for (int c = threadIdx.x; c < nrows * Q; c += kRowThreads) {
+    const int jj = c / Q;
+    if (src[jj] >= 0) dst[c] = tile[jj * QS + (c - jj * Q)];
+  }
+}
+
+__global__ void __launch_bounds__(kRowThreads) k_load_rows(const RowLayout L, const uint4 *__restrict__ rows, int64_t m,
+                                                           const int64_t *__restrict__ slot, int64_t N,
+                                                           uint64_t *__restrict__ sf, uint64_t *__restrict__ start,
+                                                           uint32_t *__restrict__ si) {
+  extern __shared__ uint4 tile[];
+  __shared__ int64_t src[kRowTile];
+  const int Q = L.bytes() / 16, QS = row_tile_chunks(L);
+  const int64_t i0 = (int64_t)blockIdx.x * kRowTile;
+  const int nenv = N - i0 < kRowTile ? (int)(N - i0) : kRowTile;
+  if (threadIdx.x < kRowTile) src[threadIdx.x] = (int)threadIdx.x < nenv ? load_source(slot, i0 + threadIdx.x, m) : -1;
+  __syncthreads();
+  // each env's row with 128-bit loads (a row is contiguous; consecutive rows too when the slots are)
+#pragma unroll 4
+  for (int c = threadIdx.x; c < nenv * Q; c += kRowThreads) {
+    const int jj = c / Q;
+    const int64_t r = src[jj];
+    if (r >= 0) tile[jj * QS + (c - jj * Q)] = rows[r * Q + (c - jj * Q)];
+  }
+  __syncthreads();
+  // scatter: lane = env of the tile, warp w takes chunks w, w + 8, ...; a masked lane stores nothing
+  const int j = threadIdx.x & 31, w = threadIdx.x >> 5;
+  if (src[j] < 0) return;
+  const int64_t i = i0 + j;
+#pragma unroll 2
+  for (int q = w; q < Q; q += kRowWarps) {
+    const uint4 c = tile[j * QS + q];
+    row_unit_put(L, sf, start, si, N, i, 2 * q, (uint64_t)c.x | ((uint64_t)c.y << 32));
+    row_unit_put(L, sf, start, si, N, i, 2 * q + 1, (uint64_t)c.z | ((uint64_t)c.w << 32));
+  }
+}
+
 }  // namespace rr
 
 // =============================================================================================
@@ -913,6 +997,44 @@ int rr_assign_balls(rr_sim *s, const int32_t *robots_host, int32_t n_robots, int
   cudaStream_t st = (cudaStream_t)stream;
   if (int jr = join_into(s, st)) return jr;
   LAUNCH_PRESET(s, st, (k_assign_balls<L>), s->k, s->sf, s->si, s->N, rl, assign_dev);
+  s->launches++;
+  CK(cudaGetLastError());
+  return RR_OK;
+}
+
+int64_t rr_snapshot_bytes_per_env(const rr_sim *s) { return s ? row_layout(s->cols, s->cfg.observer).bytes() : 0; }
+
+// The checks of rr_save_states / rr_load_states: the kernels never touch memory outside the buffers the caller described.
+static int check_rows(const rr_sim *s, const void *rows, int64_t m, const int64_t *idx, bool null_idx_ok, const char *rule) {
+  if (!s || !rows) return fail(RR_E_INVALID, "null argument");
+  if (m < 1) return fail(RR_E_INVALID, "m must be >= 1");
+  if (misaligned(rows, 16)) return fail(RR_E_INVALID, "the rows buffer must be 16-byte aligned");
+  if (misaligned(idx, 8)) return fail(RR_E_INVALID, "the index buffer must be 8-byte aligned");
+  if (!idx && !null_idx_ok) return fail(RR_E_INVALID, rule);
+  return RR_OK;
+}
+
+int rr_save_states(rr_sim *s, const int64_t *env_dev, int64_t m, void *rows_dev, void *stream) {
+  if (int rc = check_rows(s, rows_dev, m, env_dev, s && m <= s->N, "without env indices m must be <= n_envs")) return rc;
+  ON_DEVICE(s->device);
+  cudaStream_t st = (cudaStream_t)stream;
+  if (int jr = join_into(s, st)) return jr;
+  const RowLayout L = row_layout(s->cols, s->cfg.observer);
+  k_save_rows<<<(unsigned)((m + kRowTile - 1) / kRowTile), kRowThreads, row_tile_bytes(L), st>>>(
+      L, (const uint64_t *)s->sf, (const uint64_t *)s->start, (const uint32_t *)s->si, s->N, env_dev, m, (uint4 *)rows_dev);
+  s->launches++;
+  CK(cudaGetLastError());
+  return RR_OK;
+}
+
+int rr_load_states(rr_sim *s, const void *rows_dev, int64_t m, const int64_t *slot_dev, void *stream) {
+  if (int rc = check_rows(s, rows_dev, m, slot_dev, s && m == s->N, "without slot indices m must equal n_envs")) return rc;
+  ON_DEVICE(s->device);
+  cudaStream_t st = (cudaStream_t)stream;
+  if (int jr = join_into(s, st)) return jr;
+  const RowLayout L = row_layout(s->cols, s->cfg.observer);
+  k_load_rows<<<(unsigned)((s->N + kRowTile - 1) / kRowTile), kRowThreads, row_tile_bytes(L), st>>>(
+      L, (const uint4 *)rows_dev, m, slot_dev, s->N, (uint64_t *)s->sf, (uint64_t *)s->start, (uint32_t *)s->si);
   s->launches++;
   CK(cudaGetLastError());
   return RR_OK;

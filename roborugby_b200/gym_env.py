@@ -11,6 +11,8 @@ exists for API compatibility and parity tests; throughput comes from RoboRugbyVe
 of the reference (step after done, too many commands, unresolved collisions) are raised as
 `Exception` with the reference's messages.  Rendering is out of scope (SURVEY.md §2 row 12).
 """
+import copy
+
 import numpy as np
 import torch
 
@@ -183,6 +185,16 @@ class RoboRugbyEnv:
             self._v.set_starting_positions(np.asarray(lst_starting_config[0], np.float64),
                                            np.asarray(lst_starting_config[1], np.float64))
             self._v.reset_fixed(as_constructed=True)
+
+    def __deepcopy__(self, memo):
+        """copy.deepcopy(env), as planning code written against the reference branches an env: the episode goes on from
+        the same state in a new handle (RoboRugbyVecEnv.__deepcopy__: the env's saved row on the device), and the wrapper's
+        own state (TimeLimit's elapsed count, the last rewards, the views, which now look at the copy) is copied."""
+        new = object.__new__(type(self))
+        memo[id(self)] = new
+        for k, v in self.__dict__.items():
+            setattr(new, k, copy.deepcopy(v, memo))   # _v through RoboRugbyVecEnv.__deepcopy__; _elapsed, _reward, views
+        return new
 
     # -- gym.Env surface -------------------------------------------------------------------
     @property

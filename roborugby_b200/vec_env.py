@@ -59,10 +59,15 @@ class RoboRugbyVecEnv:
         _lib.check_config(cfg)   # ValueError for a reward_mask / reward_order no class composition produces, etc.
         if not torch.cuda.is_available():
             raise RuntimeError("RoboRugbyVecEnv needs a CUDA device: roborugby_b200 has no CPU fallback")
+        self._open(cfg, n_actions, pipeline)
+
+    def _open(self, cfg, n_actions, pipeline):
+        """rr_create for cfg and the handle's derived attributes (the constructor and __deepcopy__)."""
         self.cfg = cfg
         self.out_dtype = torch.float64 if cfg.out_f64 else torch.float32
         self.discrete = bool(cfg.discrete)
         dev_index = self.device.index if self.device.index is not None else torch.cuda.current_device()
+        self._dev_index = dev_index
         h = C.c_void_p()
         _lib.check(self.lib.rr_create(C.byref(cfg), self.num_envs, dev_index, C.byref(h)))
         self._h = h
@@ -80,6 +85,18 @@ class RoboRugbyVecEnv:
         self._inflight = []
         if pipeline and int(pipeline) > 1:
             self.set_pipeline(pipeline)
+
+    def __deepcopy__(self, memo):
+        """copy.deepcopy(venv): a new handle with the same rr_config and pipeline setting whose envs are loaded with every
+        env's saved row (save_states / load_states: the copy continues bit for bit, resets included) and a clone of the
+        statistics.  Output buffers are not shared and a flush buffer is not carried over."""
+        new = object.__new__(type(self))
+        memo[id(self)] = new
+        new.lib, new.env_id, new.preset, new.device, new.num_envs = self.lib, self.env_id, self.preset, self.device, self.num_envs
+        new._open(_lib.Config.from_buffer_copy(self.cfg), self.n_actions, self.pipeline)
+        new.load_states(self.save_states())
+        new.stats.copy_(self.stats)
+        return new
 
     # ------------------------------------------------------------------ sub-batch pipeline
     def set_pipeline(self, sub_batches):
@@ -344,6 +361,73 @@ class RoboRugbyVecEnv:
         step = np.ascontiguousarray(st["step"], np.int32).reshape(N)
         p = lambda a: a.ctypes.data_as(C.c_void_p)
         _lib.check(self.lib.rr_set_state(self._h, p(rob), p(rhist), p(rflag), p(ball), p(step)))
+
+    # ------------------------------------------------------------------ saved states on the device
+    @property
+    def state_row_bytes(self):
+        """S: the width in bytes of one saved env row (rr_snapshot_bytes_per_env); it identifies the row layout."""
+        return int(self.lib.rr_snapshot_bytes_per_env(self._h))
+
+    def _indices(self, idx, n, bound, what):
+        """idx as a contiguous int64 tensor on the env's device; ValueError unless it is an integer tensor [n] (n None: any
+        length), IndexError, before anything is launched, for an entry >= bound and, for env indices, one < 0 (a negative
+        slot keeps its env).  The check is one reduction, and for a device tensor one synchronisation."""
+        if not torch.is_tensor(idx) or idx.dtype.is_floating_point or idx.dtype == torch.bool or idx.dim() != 1 or (
+                n is not None and idx.numel() != n):
+            raise ValueError(f"{what} must be an integer tensor [{'m' if n is None else n}]")
+        bad = (idx >= bound) | (idx < 0) if what == "envs" else idx >= bound
+        if bool(bad.any()):
+            raise IndexError(f"{what} entries must be " + (f"in [0, {bound})" if what == "envs" else f"< {bound}"))
+        return idx.to(self.device, torch.int64).contiguous()
+
+    def save_states(self, envs=None, out=None):
+        """Save env states on the device (rr_save_states): returns a contiguous uint8 tensor [m, state_row_bytes] on the
+        env's device whose row j is env envs[j] (envs: int tensor [m], duplicates allowed; None: every env in order).
+        `out` reuses a caller tensor of that shape.  Stream-ordered on the current stream; joins the sub-batch pipeline
+        first, so it sees every step issued before it."""
+        S = self.state_row_bytes
+        ep = None
+        if envs is not None:
+            envs = self._indices(envs, None, self.num_envs, "envs")
+            ep = envs.data_ptr()
+        m = self.num_envs if envs is None else envs.numel()
+        if m < 1:
+            raise ValueError("nothing to save: envs is empty")
+        if out is None:
+            out = torch.empty(m, S, dtype=torch.uint8, device=self.device)
+        else:
+            self._check_rows(out, m)
+        _lib.check(self.lib.rr_save_states(self._h, ep, m, out.data_ptr(), self._stream()))
+        return out
+
+    def load_states(self, rows, slots=None):
+        """Load saved rows into the envs on the device (rr_load_states): env i receives rows[slots[i]] (slots: int tensor
+        [num_envs]; a negative entry keeps env i; None: env i receives rows[i], and rows has num_envs rows).  rows: a
+        contiguous uint8 tensor [m, state_row_bytes] on the env's device, from save_states of this or any handle with the
+        same row width.  Every entry point then reports for env i what it reported for the saved env, and stepping it
+        continues the saved env bit for bit until a random reset, which draws with env i's own global index.  The
+        statistics are not touched.  Stream-ordered on the current stream, like save_states."""
+        if not torch.is_tensor(rows) or rows.dim() != 2:
+            raise ValueError("rows must be a uint8 tensor [m, state_row_bytes]")
+        m = rows.shape[0]
+        self._check_rows(rows, m)
+        sp = None
+        if slots is not None:
+            slots = self._indices(slots, self.num_envs, m, "slots")
+            sp = slots.data_ptr()
+        elif m != self.num_envs:
+            raise ValueError(f"without slots rows must have num_envs = {self.num_envs} rows, got {m}")
+        _lib.check(self.lib.rr_load_states(self._h, rows.data_ptr(), m, sp, self._stream()))
+
+    def _check_rows(self, rows, m):
+        S = self.state_row_bytes
+        if rows.dtype != torch.uint8 or tuple(rows.shape) != (m, S) or m < 1:
+            raise ValueError(f"rows must be uint8 [{m}, {S}] (state_row_bytes of this env), got {rows.dtype} "
+                             f"{tuple(rows.shape)}")
+        if rows.device.type != "cuda" or rows.device.index != self._dev_index:
+            raise ValueError(f"rows must be on {self.device}, got {rows.device}")
+        if not rows.is_contiguous() or rows.data_ptr() % 16:
+            raise ValueError("rows must be contiguous and 16-byte aligned")
 
     def goal_state(self):
         """Goal bookkeeping (goal_scoring=True): dict of numpy arrays alive [N, B] (0/1), score [N, 2] (happy goal,
