@@ -361,7 +361,13 @@ int64_t rr_state_bytes_per_env(const rr_sim *s);
  * counterpart: the reference uses CPython's float division and libm).  which 0: the branch-free fp64 division
  * of the contact paths (rr_sim.cuh div_core) against the compiler's division on >= n random operand pairs.
  * out2[0] = results that differ although the routine reported the operands in range (must be 0),
- * out2[1] = operand pairs it reported out of range (those are redone with the ordinary division). */
+ * out2[1] = operand pairs it reported out of range (those are redone with the ordinary division).
+ * which 1: the branch-free side x line block of the contact paths (rr_sim.cuh sides_x_lines on the device) against
+ * the ordinary pair-after-pair evaluation (sides_x_lines_plain), both on the device, on >= n inputs: half shaped like
+ * the simulator's (robot corners and ball diameters of a GAME env), half adversarial (parallel, vertical, horizontal
+ * and zero-length lines, lines through corners, huge and tiny coordinates, NaN and infinity).
+ * out2[0] = inputs on which the mask, an intersection point, a slope, an intercept or the error bits differ (must
+ * be 0), out2[1] = inputs on which the block fell back to the ordinary divisions. */
 int rr_selftest(int device, int which, int64_t n, uint64_t seed, int64_t *out2);
 
 #ifdef __cplusplus

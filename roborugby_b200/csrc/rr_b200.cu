@@ -817,6 +817,135 @@ __global__ void k_selftest_div(uint64_t seed, int64_t per_thread, unsigned long 
   atomicAdd(&out[0], bad);
   atomicAdd(&out[1], flagged);
 }
+
+__device__ __forceinline__ double unit_double(uint64_t &st) { return (double)(splitmix64(st) >> 11) * 0x1p-53; }
+__device__ __forceinline__ bool same_value(double a, double b) {  // bit-identical, or both NaN
+  return (isnan(a) && isnan(b)) || __double_as_longlong(a) == __double_as_longlong(b);
+}
+
+// which 1: the branch-free side x line block of sides_x_lines (the __CUDA_ARCH__ branch) against sides_x_lines_plain, both
+// on the device.  Half of the inputs are shaped like the simulator's: robot 0 of a GAME Env bound the way k_step binds
+// it (trig table and hot fields in dynamic shared memory), its centre in the arena, its heading on the 0.2-degree grid
+// plus rounding drift (exactly 0 / 90 / 180 / 270 and one ulp either side of them now and then), the ball anywhere
+// within contact distance (exactly on a corner or a side midpoint now and then), and the ball's diameters as
+// ball_robot_collided (buf 0) and apply_force_to_ball (buf 0.5) build them.  The other half are adversarial: lines
+// parallel to a side (exact den == 0), vertical / horizontal and zero-length lines, lines through a corner, huge and
+// tiny coordinates, NaN and infinity.  out[0] = inputs on which the mask, a point, a slope, an intercept or the error
+// bits differ (must be 0), out[1] = inputs on which the block fell back to the ordinary divisions.
+__global__ void __launch_bounds__(128, 1) k_selftest_sides(const __grid_constant__ Consts k, uint64_t seed,
+                                                           int64_t per_thread, unsigned long long *out) {
+  using E = LGame::E;
+  E e;
+  double cold[E::kColdDoubles];
+  e.trig = stage_trig_table();
+  bind_env(e, cold);
+  e.rrot(0) = rr_nan();  // no heading yet, and no inner-corner offsets cached for one
+  e.rc(0, 3) = rr_nan();
+  uint64_t st = seed ^ (0x9E6C63D0676A9A99ull * (uint64_t)(blockIdx.x * blockDim.x + threadIdx.x + 1));
+  unsigned long long bad = 0, fell = 0;
+  for (int64_t it = 0; it < per_thread; it++) {
+    P2 rc[4];
+    Seg ln[2];
+    double buf = 0.0;
+    if ((it & 1) == 0) {  // simulator-shaped
+      const uint64_t sel = splitmix64(st);
+      double rot = 0.2 * (double)(int)(sel % 1800u);
+      switch ((sel >> 12) % 8) {
+        case 0: break;                                                         // on the grid
+        case 1: rot += (unit_double(st) - 0.5) * 1e-11; break;                 // accumulated drift
+        case 2: rot = 90.0 * (double)(int)((sel >> 20) % 4u); break;           // axis-aligned
+        case 3: rot = nextafter(90.0 * (double)(int)((sel >> 20) % 4u) + (((sel >> 22) & 1) ? 0.0 : 360.0),
+                                ((sel >> 22) & 1) ? 400.0 : 0.0) ; break;      // one ulp off an axis
+        default: rot += (double)((int)((sel >> 20) % 7u) - 3) * 1e-13; break;  // a few ulps of drift
+      }
+      rot = norm_rot(rot);
+      e.rcx(0) = 30.0 + 740.0 * unit_double(st);
+      e.rcy(0) = 30.0 + 740.0 * unit_double(st);
+      if (!(e.rrot(0) == rot)) {
+        e.rrot(0) = rot;
+        robot_refresh_corners(e, k, 0);
+      }
+      robot_refresh_ltrb(e, 0);
+      robot_corners(e, 0, rc);
+      double bx, by;
+      const uint64_t where = splitmix64(st) % 16u;
+      if (where < 4) {  // on a corner
+        bx = rc[where].x; by = rc[where].y;
+      } else if (where < 8) {  // on a side midpoint
+        const Seg s = side_from_corners(rc, (int)where - 4);
+        bx = (s.a.x + s.b.x) / 2.0; by = (s.a.y + s.b.y) / 2.0;
+      } else {  // anywhere within 7.5 px of the robot, in its own frame
+        const double u = (unit_double(st) * 2.0 - 1.0) * 17.5, v = (unit_double(st) * 2.0 - 1.0) * 27.5;
+        const double ax = (e.ktrx(0) + e.kbrx(0)) * 0.5, ay = (e.ktry(0) + e.kbry(0)) * 0.5;  // half-length axis
+        const double wx = (e.kbrx(0) - e.ktrx(0)) * 0.5, wy = (e.kbry(0) - e.ktry(0)) * 0.5;  // half-width axis
+        bx = e.rcx(0) + u * 0.1 * ax + v * 0.05 * wx;
+        by = e.rcy(0) + u * 0.1 * ay + v * 0.05 * wy;
+      }
+      P2 ic[4];
+      inner_corners(e, k, 0, bx, by, ic);
+      if ((sel >> 30) & 1) {  // ball_robot_collided
+        ln[0] = Seg{ic[0], ic[3]}; ln[1] = Seg{ic[1], ic[2]};
+      } else {  // apply_force_to_ball, bounce_ball_off_bot (with buf 0)
+        ln[0] = Seg{ic[2], ic[1]}; ln[1] = Seg{ic[3], ic[0]};
+        buf = ((sel >> 31) & 1) ? 0.5 : 0.0;
+      }
+    } else {  // adversarial: a rect with small integer corner offsets, so that parallel lines have equal slopes exactly
+      const uint64_t sel = splitmix64(st);
+      const double cx = (double)(int)(sel % 700u) + 50.0, cy = (double)(int)((sel >> 10) % 700u) + 50.0;
+      const double px = (double)((int)((sel >> 20) % 41u) - 20), py = (double)((int)((sel >> 26) % 41u) - 20);
+      const double qx = -py, qy = px;  // a perpendicular axis of the same length (a square, possibly degenerate)
+      rc[0] = P2{cx - px - qx, cy - py - qy}; rc[1] = P2{cx + px - qx, cy + py - qy};
+      rc[2] = P2{cx - px + qx, cy - py + qy}; rc[3] = P2{cx + px + qx, cy + py + qy};
+      buf = ((sel >> 32) & 1) ? 0.5 : 0.0;
+      for (int q = 0; q < 2; q++) {
+        const uint64_t h = splitmix64(st);
+        const double ox = (double)((int)(h % 61u) - 30), oy = (double)((int)((h >> 8) % 61u) - 30);
+        const P2 a{cx + ox, cy + oy};
+        const Seg sd = side_from_corners(rc, (int)((h >> 16) % 4u));
+        const P2 cn = rc[(h >> 18) % 4u];
+        switch ((h >> 20) % 8) {
+          case 0: ln[q] = Seg{P2{sd.a.x + ox, sd.a.y + oy}, P2{sd.b.x + ox, sd.b.y + oy}}; break;  // parallel to a side
+          case 1: ln[q] = Seg{a, P2{a.x, a.y + 9.0}}; break;                                          // vertical
+          case 2: ln[q] = Seg{a, P2{a.x - 9.0, a.y}}; break;                                          // horizontal
+          case 3: ln[q] = Seg{a, a}; break;                                                            // zero length
+          case 4: ln[q] = Seg{cn, a}; break;                                                           // through a corner
+          case 5: ln[q] = Seg{sd.a, sd.b}; break;                                                      // along a side
+          default: ln[q] = Seg{a, P2{cx - ox + (double)((int)((h >> 24) % 7u) - 3), cy - oy}}; break;  // across
+        }
+      }
+      const uint64_t mod = splitmix64(st) % 16u;
+      if (mod < 6) {  // the same geometry scaled to huge or tiny coordinates
+        const double f = mod == 0 ? 0x1p+900 : mod == 1 ? 0x1p-900 : mod == 2 ? 0x1p+500 : mod == 3 ? 0x1p-1000 : mod == 4 ? 1e-310 : 0x1p+1000;
+        for (int i = 0; i < 4; i++) { rc[i].x *= f; rc[i].y *= f; }
+        for (int q = 0; q < 2; q++) { ln[q].a.x *= f; ln[q].a.y *= f; ln[q].b.x *= f; ln[q].b.y *= f; }
+      } else if (mod == 6 || mod == 7) {  // a NaN or an infinity in one coordinate
+        const double v = mod == 6 ? rr_nan() : HUGE_VAL;
+        const uint64_t c = splitmix64(st) % 12u;
+        if (c < 8) { if (c & 1) rc[c >> 1].y = v; else rc[c >> 1].x = v; }
+        else if (c == 8) ln[0].a.x = v; else if (c == 9) ln[0].b.y = v; else if (c == 10) ln[1].a.y = v; else ln[1].b.x = v;
+      } else if (mod == 8) {  // arbitrary doubles
+        for (int i = 0; i < 4; i++) { rc[i].x = random_double(st, 40); rc[i].y = random_double(st, 40); }
+        for (int q = 0; q < 2; q++) {
+          ln[q].a.x = random_double(st, 40); ln[q].a.y = random_double(st, 40);
+          ln[q].b.x = random_double(st, 40); ln[q].b.y = random_double(st, 40);
+        }
+      }
+    }
+    P2 pt[8], pt2[8];
+    double lm[2], lb[2], lm2[2], lb2[2];
+    unsigned err = 0, err2 = 0;
+    bool fb = false;
+    const unsigned mask = sides_x_lines(rc, ln, buf, pt, lm, lb, err, &fb);
+    const unsigned mask2 = sides_x_lines_plain(rc, ln, buf, pt2, lm2, lb2, err2);
+    bool same = mask == mask2 && err == err2;
+    for (int i = 0; i < 8; i++) same = same && same_value(pt[i].x, pt2[i].x) && same_value(pt[i].y, pt2[i].y);
+    for (int q = 0; q < 2; q++) same = same && same_value(lm[q], lm2[q]) && same_value(lb[q], lb2[q]);
+    bad += same ? 0 : 1;
+    fell += fb ? 1 : 0;
+  }
+  atomicAdd(&out[0], bad);
+  atomicAdd(&out[1], fell);
+}
 }  // namespace rr
 
 int rr_selftest(int device, int which, int64_t n, uint64_t seed, int64_t *out2) {
@@ -825,10 +954,21 @@ int rr_selftest(int device, int which, int64_t n, uint64_t seed, int64_t *out2) 
   unsigned long long *d = nullptr;
   CK(cudaMalloc(&d, 2 * sizeof(unsigned long long)));
   CK(cudaMemset(d, 0, 2 * sizeof(unsigned long long)));
-  const int blocks = 148 * 4, threads = 256;
+  const int blocks = 148 * 4, threads = which == 1 ? 128 : 256;
   const int64_t per_thread = (n + (int64_t)blocks * threads - 1) / ((int64_t)blocks * threads);
-  if (which == 0) rr::k_selftest_div<<<blocks, threads>>>(seed, per_thread, d);
-  else { cudaFree(d); return fail(RR_E_INVALID, "unknown selftest"); }
+  if (which == 0) {
+    rr::k_selftest_div<<<blocks, threads>>>(seed, per_thread, d);
+  } else if (which == 1) {
+    rr_config cfg;
+    rr_default_config(&cfg, RR_PRESET_GAME, "RoboRugbySimpleDuel-v2");
+    const size_t sm = LGame::smem_bytes(threads);
+    cudaError_t ae = cudaFuncSetAttribute(rr::k_selftest_sides, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
+    if (ae != cudaSuccess) { cudaFree(d); CK(ae); }
+    rr::k_selftest_sides<<<blocks, threads, sm>>>(make_consts(cfg), seed, per_thread, d);
+  } else {
+    cudaFree(d);
+    return fail(RR_E_INVALID, "unknown selftest");
+  }
   cudaError_t e = cudaDeviceSynchronize();
   unsigned long long h[2] = {0, 0};
   if (e == cudaSuccess) e = cudaMemcpy(h, d, sizeof h, cudaMemcpyDeviceToHost);
