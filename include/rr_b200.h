@@ -318,6 +318,48 @@ int64_t rr_snapshot_bytes_per_env(const rr_sim *s);
 int rr_save_states(rr_sim *s, const int64_t *env_dev, int64_t m, void *rows_dev, void *stream);
 int rr_load_states(rr_sim *s, const void *rows_dev, int64_t m, const int64_t *slot_dev, void *stream);
 
+/* A reset pool: saved rows that auto-reset may start episodes from (rr_step_pool); archived-state curricula such as
+ * "return to a cell, then explore", starts at states where an agent keeps failing, or a late-game start distribution. */
+typedef struct rr_reset_pool {
+  const void *rows_dev;  /* m rows of rr_snapshot_bytes_per_env(s) bytes (rr_save_states of any handle of that width),
+                            16-byte aligned */
+  int64_t m;             /* 1 <= m <= INT32_MAX */
+  const double *cdf_dev; /* NULL: every slot equally likely; else m non-decreasing doubles with cdf[m-1] > 0, the
+                            inclusive prefix sum of the slots' weights, 8-byte aligned */
+  double p_pool;         /* probability that a reset takes a pool row, in [0, 1]; 1 = always */
+} rr_reset_pool;
+
+/* rr_step_info whose auto-resets may start the next episode from a row of a reset pool, inside the fused launch.
+ * With pool == NULL this is rr_step_info and runs the same kernels.  On a launch with a pool, every row that reports
+ * done = 1 (auto_reset) resets its env as follows:
+ *   1. the episode counter is incremented, as by every auto-reset;
+ *   2. one Philox4x32-10 block, key = cfg.seed, counter = (global env index (two words), the new episode counter,
+ *      0xFFFFFFFF), gives words w0..w3 and u0 = (w0 << 32 | w1) >> 11 over 2^53, u1 likewise from w2, w3.  u0 < p_pool
+ *      takes a pool row, otherwise the reset is random.  u1 picks the slot: without cdf min(floor(u1 m), m - 1), with cdf
+ *      the smallest j with u1 cdf[m-1] < cdf[j], so a zero-weight slot is never drawn.  The draw depends on the seed,
+ *      the global index and the episode only, not on env_offset sharding, the sub-batch pipeline or k_steps;
+ *   3. random: the reset rr_step makes (rr_reset's placement);
+ *   4. pool: the env becomes what rr_load_states makes of the row, except that the episode counter keeps the value of
+ *      step 1 instead of the row's (otherwise envs reset from one row would draw the same next slot for ever).
+ *      Everything else comes from the row: robots, balls, returns, step counter, sticky error mask, last naughty count,
+ *      goal words, prior-step poses, the episode-counted bit, and the starting layout (rr_reset_fixed and
+ *      rr_get_starting_positions then use the row's layout).
+ * The rest of the launch steps the loaded state.  The done row's obs is the observation of the state after the reset;
+ * its final observation and row_flags describe the state before it, as in rr_step_info.  The statistics follow
+ * rr_get_stats: the episode-counted bit travels with the row, so an episode continued from a row is counted once when it
+ * ends, with the row's return and length plus what follows.  A row saved from a finished episode is refused with
+ * RR_ERR_STEP_AFTER_DONE on its next step and reset again: legal, and at most one reset per env-step.
+ *   reset_slot_dev  int32 [K][N], optional, written on every row: the slot the row's reset loaded, or -1 (no reset, or a
+ *                   random one; all -1 without a pool).  128-bit stores when 16-byte aligned and N is a multiple of 4.
+ * RR_E_INVALID, nothing launched: rr_step_info's argument errors; a NULL rows_dev; m outside [1, INT32_MAX]; rows_dev not
+ * 16-byte or cdf_dev not 8-byte aligned; p_pool outside [0, 1] or NaN; a pool on a handle with auto_reset = 0;
+ * reset_slot_dev not 4-byte aligned.  The kernel cannot check the row width or the cdf's contents: rows of another width
+ * give a wrong state, and a malformed cdf can pick a wrong slot but never one outside [0, m).  The kernels read the pool
+ * while they run: with a sub-batch pipeline keep its memory unchanged until the groups have run, as for the actions. */
+int rr_step_pool(rr_sim *s, const void *actions_dev, int32_t n_actions, int32_t k_steps, void *obs_h_dev,
+                 void *obs_g_dev, void *rew_dev, uint8_t *done_dev, void *final_obs_h_dev, void *final_obs_g_dev,
+                 uint8_t *row_flags_dev, const rr_reset_pool *pool, int32_t *reset_slot_dev, void *stream);
+
 /* Goal bookkeeping (goal_scoring = 1) to HOST; any pointer may be NULL.  alive[N]: bit b = ball b still in play;
  * score[N][2]: Goal.get_score() of the happy and the grumpy goal (RR_Goal.py:87-88); destroyed[N]: bit 0 happy goal,
  * bit 1 grumpy goal (Goal.is_destroyed, :90-91); dwell[N][2][B]: steps ball b has stayed inside that goal's triangle

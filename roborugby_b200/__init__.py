@@ -10,9 +10,9 @@ from .stats import allreduce_stats, shard_envs, summarize  # noqa: F401
 
 
 def __getattr__(name):  # torch-dependent modules are imported lazily
-    if name in ("RoboRugbyVecEnv",):
-        from .vec_env import RoboRugbyVecEnv
-        return RoboRugbyVecEnv
+    if name in ("RoboRugbyVecEnv", "ResetPool"):
+        from . import vec_env
+        return getattr(vec_env, name)
     if name in ("og_twitchy_actions",):
         from .players import og_twitchy_actions
         return og_twitchy_actions

@@ -44,6 +44,11 @@ class Config(C.Structure):
     ]
 
 
+class ResetPoolC(C.Structure):
+    """struct rr_reset_pool (include/rr_b200.h)."""
+    _fields_ = [("rows_dev", C.c_void_p), ("m", C.c_int64), ("cdf_dev", C.c_void_p), ("p_pool", C.c_double)]
+
+
 # name -> (restype, argtypes); kept in one table so tests can check it against the header
 _vp, _i32, _i64 = C.c_void_p, C.c_int32, C.c_int64
 SIGNATURES = {
@@ -77,6 +82,7 @@ SIGNATURES = {
     "rr_snapshot_bytes_per_env": (_i64, [_vp]),
     "rr_save_states": (C.c_int, [_vp, _vp, _i64, _vp, _vp]),
     "rr_load_states": (C.c_int, [_vp, _vp, _i64, _vp, _vp]),
+    "rr_step_pool": (C.c_int, [_vp, _vp, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, C.POINTER(ResetPoolC), _vp, _vp]),
     "rr_goal_state": (C.c_int, [_vp, _vp, _vp, _vp, _vp]),
     "rr_error_mask": (C.c_int, [_vp, _vp, _i32]),
     "rr_last_naughty": (C.c_int, [_vp, _vp]),

@@ -17,6 +17,7 @@
 #include <cstring>
 #include <new>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include "rr_sim.cuh"
@@ -143,6 +144,13 @@ struct StepArgs {
   void *final_obs_h, *final_obs_g;  // rr_step_info: out_t [K][N][D], written on done rows only (k_step<L, OutT, true>)
   uint8_t *row_flags;               // rr_step_info: RR_ROW_* [K][N]
 };
+// rr_step_pool (k_step<L, OutT, true, true>): the pool, the handle's start columns its resets write, and the slot rows.
+// A struct of its own, so that the other variants keep their parameter block.
+struct PoolStepArgs : StepArgs {
+  double *start;        // [3R + 2B][N]
+  ResetPool pool;
+  int32_t *reset_slot;  // [K][N] or NULL; vec bit 5: its rows can be written with 128-bit stores
+};
 
 __device__ __forceinline__ double warp_sum(double v) {
 #pragma unroll
@@ -154,8 +162,11 @@ __device__ __forceinline__ double warp_sum(double v) {
 // last block (i >= N) run the control flow without an env so that the per-frame barrier is uniform.
 // INFO: also report every row's RR_ROW_* flags and, on done rows, the terminal observation taken before the auto-reset
 // (rr_step_info).  A template switch, not a run-time branch: the default kernels keep their registers and stack.
-template <class L, typename OutT, bool INFO = false>
-__global__ void __launch_bounds__(L::kMaxBlock, L::kStepBlocksPerSM) k_step(const __grid_constant__ Consts k, const __grid_constant__ StepArgs a) {
+// POOL (with INFO): a done row's auto-reset may load a row of a reset pool instead (rr_step_pool, pool_reset).
+template <class L, typename OutT, bool INFO = false, bool POOL = false>
+__global__ void __launch_bounds__(L::kMaxBlock, L::kStepBlocksPerSM) k_step(const __grid_constant__ Consts k,
+    const __grid_constant__ typename std::conditional<POOL, PoolStepArgs, StepArgs>::type a) {
+  static_assert(INFO || !POOL, "the pool variant reports rr_step_info's outputs as well");
   using E = typename L::E;
   constexpr int R = E::R;
   const int64_t i = ((int64_t)a.block0 + blockIdx.x) * blockDim.x + threadIdx.x;
@@ -231,7 +242,12 @@ __global__ void __launch_bounds__(L::kMaxBlock, L::kStepBlocksPerSM) k_step(cons
         }
       }
     }
-    if (live) step_auto_reset(e, k, done_flag, (uint64_t)(k.env_offset + i));
+    int32_t slot = -1;
+    if constexpr (POOL) {
+      if (live) slot = step_pool_auto_reset(e, k, done_flag, (uint64_t)(k.env_offset + i), a.pool, a.start + i, a.N, last_naughty);
+    } else {
+      if (live) step_auto_reset(e, k, done_flag, (uint64_t)(k.env_offset + i));
+    }
     // Results: written once, never read back by this launch.  Every warp turns its 32 rows of each buffer into
     // coalesced 128-bit streaming stores (warp_store_rows); all lanes of the warp take part (no divergence here).
     {
@@ -251,6 +267,12 @@ __global__ void __launch_bounds__(L::kMaxBlock, L::kStepBlocksPerSM) k_step(cons
         if (a.row_flags) {
           const unsigned char rf[1] = {row_flag};
           warp_store_rows<unsigned char>(a.row_flags + row0, rf, 1, live, full && (a.vec & 16u), stage, lane);
+        }
+      }
+      if constexpr (POOL) {
+        if (a.reset_slot) {
+          const int32_t rs[1] = {slot};
+          warp_store_rows<int32_t>(a.reset_slot + row0, rs, 1, live, full && (a.vec & 32u), stage, lane);
         }
       }
       if (dim > 0 && (a.obs_h || a.obs_g)) {
@@ -626,6 +648,7 @@ static cudaError_t opt_in_shared_memory() {
     if (e == cudaSuccess) e = r;
   };
   set(k_step<L, float>); set(k_step<L, double>); set(k_step<L, float, true>); set(k_step<L, double, true>);
+  set(k_step<L, float, true, true>); set(k_step<L, double, true, true>);
   set(k_init<L>); set(k_reset<L>); set(k_reset_fixed<L>);
   set(k_observe<L, float>); set(k_observe<L, double>);
   set(k_observe_entity<L, float>); set(k_observe_entity<L, double>); set(k_assign_balls<L>);
@@ -711,9 +734,11 @@ int rr_create(const rr_config *cfg, int64_t n_envs, int device, rr_sim **out) {
     if (cfg->goal_scoring) {
       set(k_step<LGameGoalsWide, float>); set(k_step<LGameGoalsWide, double>);
       set(k_step<LGameGoalsWide, float, true>); set(k_step<LGameGoalsWide, double, true>);
+      set(k_step<LGameGoalsWide, float, true, true>); set(k_step<LGameGoalsWide, double, true, true>);
     } else {
       set(k_step<LGameWide, float>); set(k_step<LGameWide, double>);
       set(k_step<LGameWide, float, true>); set(k_step<LGameWide, double, true>);
+      set(k_step<LGameWide, float, true, true>); set(k_step<LGameWide, double, true, true>);
     }
     if (we != cudaSuccess) { rr_destroy(s); return fail(RR_E_CUDA, std::string("cudaFuncSetAttribute: ") + cudaGetErrorString(we)); }
   }
@@ -1196,8 +1221,10 @@ int rr_step(rr_sim *s, const void *actions, int32_t n_actions, int32_t k_steps, 
   return rr_step_info(s, actions, n_actions, k_steps, obs_h, obs_g, rew, done, nullptr, nullptr, nullptr, stream);
 }
 
-int rr_step_info(rr_sim *s, const void *actions, int32_t n_actions, int32_t k_steps, void *obs_h, void *obs_g, void *rew,
-                 uint8_t *done, void *final_obs_h, void *final_obs_g, uint8_t *row_flags, void *stream) {
+// rr_step_info, and rr_step_pool when `pool` is given (its checks made by the caller)
+static int step_launch(rr_sim *s, const void *actions, int32_t n_actions, int32_t k_steps, void *obs_h, void *obs_g,
+                       void *rew, uint8_t *done, void *final_obs_h, void *final_obs_g, uint8_t *row_flags,
+                       const rr_reset_pool *pool, int32_t *reset_slot, void *stream) {
   if (!s) return fail(RR_E_INVALID, "null handle");
   int rc = check_actions(s, n_actions, k_steps);
   if (rc) return rc;
@@ -1208,7 +1235,8 @@ int rr_step_info(rr_sim *s, const void *actions, int32_t n_actions, int32_t k_st
   if (rr_obs_dim(s) == 0) final_obs_h = final_obs_g = nullptr;  // no observation: nothing to report
   if (misaligned(final_obs_h, osz) || misaligned(final_obs_g, osz))
     return fail(RR_E_INVALID, "final observation buffers must be aligned to their element type");
-  const bool info = final_obs_h || final_obs_g || row_flags;
+  const bool pooled = pool != nullptr;
+  const bool info = pooled || final_obs_h || final_obs_g || row_flags;
   ON_DEVICE(s->device);
   cudaStream_t st = (cudaStream_t)stream;
   Consts k = s->k;
@@ -1222,7 +1250,13 @@ int rr_step_info(rr_sim *s, const void *actions, int32_t n_actions, int32_t k_st
   if (rows16(done, (size_t)s->N)) vec |= 4u;
   if ((((uintptr_t)actions) & 3u) == 0) vec |= 8u;
   if (rows16(row_flags, (size_t)s->N)) vec |= 16u;
-  StepArgs a{s->sf, s->si, s->stats, actions, obs_h, obs_g, rew, done, s->N, k_steps, vec, 0, final_obs_h, final_obs_g, row_flags};
+  if (rows16(reset_slot, (size_t)s->N * 4)) vec |= 32u;
+  PoolStepArgs pa{};
+  if (pooled) pa.pool = ResetPool{(const uint64_t *)pool->rows_dev, pool->cdf_dev, pool->m, pool->p_pool};
+  pa.start = s->start;
+  pa.reset_slot = reset_slot;
+  StepArgs &a = pa;  // what the other variants take
+  a = StepArgs{s->sf, s->si, s->stats, actions, obs_h, obs_g, rew, done, s->N, k_steps, vec, 0, final_obs_h, final_obs_g, row_flags};
   const bool game = s->cfg.preset == RR_PRESET_GAME, goals = s->cfg.goal_scoring != 0, f64 = s->cfg.out_f64 != 0;
   // one stream-ordered launch per call over more envs than 384-thread blocks cover in one wave: 448-thread blocks
   const bool wide = game && s->pipe <= 1 && (s->N + LGame::kMaxBlock - 1) / LGame::kMaxBlock > s->sms &&
@@ -1234,7 +1268,9 @@ int rr_step_info(rr_sim *s, const void *actions, int32_t n_actions, int32_t k_st
 #define RR_STEP_CASE(LTYPE)                                                                                  \
     do {                                                                                                     \
       const size_t sm = LTYPE::smem_bytes(blk);                                                              \
-      if (info && f64) k_step<LTYPE, double, true><<<(unsigned)nblocks, blk, sm, on>>>(k, a);                \
+      if (pooled && f64) k_step<LTYPE, double, true, true><<<(unsigned)nblocks, blk, sm, on>>>(k, pa);       \
+      else if (pooled) k_step<LTYPE, float, true, true><<<(unsigned)nblocks, blk, sm, on>>>(k, pa);          \
+      else if (info && f64) k_step<LTYPE, double, true><<<(unsigned)nblocks, blk, sm, on>>>(k, a);           \
       else if (info) k_step<LTYPE, float, true><<<(unsigned)nblocks, blk, sm, on>>>(k, a);                   \
       else if (f64) k_step<LTYPE, double><<<(unsigned)nblocks, blk, sm, on>>>(k, a);                         \
       else k_step<LTYPE, float><<<(unsigned)nblocks, blk, sm, on>>>(k, a);                                   \
@@ -1269,6 +1305,34 @@ int rr_step_info(rr_sim *s, const void *actions, int32_t n_actions, int32_t k_st
     s->pipe_pending = true;
   }
   CK(cudaGetLastError());
+  return RR_OK;
+}
+
+int rr_step_info(rr_sim *s, const void *actions, int32_t n_actions, int32_t k_steps, void *obs_h, void *obs_g, void *rew,
+                 uint8_t *done, void *final_obs_h, void *final_obs_g, uint8_t *row_flags, void *stream) {
+  return step_launch(s, actions, n_actions, k_steps, obs_h, obs_g, rew, done, final_obs_h, final_obs_g, row_flags, nullptr,
+                     nullptr, stream);
+}
+
+int rr_step_pool(rr_sim *s, const void *actions, int32_t n_actions, int32_t k_steps, void *obs_h, void *obs_g, void *rew,
+                 uint8_t *done, void *final_obs_h, void *final_obs_g, uint8_t *row_flags, const rr_reset_pool *pool,
+                 int32_t *reset_slot, void *stream) {
+  if (!s) return fail(RR_E_INVALID, "null handle");
+  if (pool) {
+    if (!pool->rows_dev) return fail(RR_E_INVALID, "reset pool: rows_dev is null");
+    if (pool->m < 1 || pool->m > INT32_MAX) return fail(RR_E_INVALID, "reset pool: m must be in [1, INT32_MAX]");
+    if (misaligned(pool->rows_dev, 16)) return fail(RR_E_INVALID, "reset pool: rows_dev must be 16-byte aligned");
+    if (misaligned(pool->cdf_dev, 8)) return fail(RR_E_INVALID, "reset pool: cdf_dev must be 8-byte aligned");
+    if (!(pool->p_pool >= 0.0 && pool->p_pool <= 1.0)) return fail(RR_E_INVALID, "reset pool: p_pool must lie in [0, 1]");
+    if (!s->cfg.auto_reset) return fail(RR_E_INVALID, "reset pool: the handle was created with auto_reset = 0");
+  }
+  if (misaligned(reset_slot, 4)) return fail(RR_E_INVALID, "reset_slot must be 4-byte aligned");
+  const int rc = step_launch(s, actions, n_actions, k_steps, obs_h, obs_g, rew, done, final_obs_h, final_obs_g, row_flags,
+                             pool, reset_slot, stream);
+  if (rc || pool || !reset_slot) return rc;
+  // without a pool these are rr_step_info's kernels, and no row is reset from a pool
+  ON_DEVICE(s->device);
+  CK(cudaMemsetAsync(reset_slot, 0xff, sizeof(int32_t) * (size_t)k_steps * (size_t)s->N, (cudaStream_t)stream));
   return RR_OK;
 }
 

@@ -22,6 +22,48 @@ from . import _lib
 from .constants import ENV_IDS, get_preset
 
 
+class ResetPool:
+    """Saved env rows that auto-reset may start episodes from (rr_step_pool): pass it to step_k / step as reset_pool.
+
+    rows: a contiguous, 16-byte aligned uint8 CUDA tensor [m, S] from save_states of any env with row width S.
+    weights: None (every slot equally likely) or m finite, non-negative numbers with a positive sum; a zero-weight slot
+    is never drawn.  p: the probability that a reset takes a pool row rather than a random placement.
+    The weights are checked with one synchronisation and turned into an fp64 prefix sum on the rows' device.  The pool
+    keeps references to rows and that prefix sum: the kernels read them while they run, so do not change them in place
+    while a launch with the pool may still run."""
+
+    def __init__(self, rows, weights=None, p=1.0):
+        if not torch.is_tensor(rows) or rows.dtype != torch.uint8 or rows.dim() != 2 or rows.shape[0] < 1:
+            raise ValueError("rows must be a uint8 tensor [m, S] with m >= 1 (save_states)")
+        m = rows.shape[0]
+        if m > 0x7FFFFFFF:
+            raise ValueError(f"a reset pool holds at most 2^31 - 1 rows, got {m}")
+        p = float(p)
+        if not 0.0 <= p <= 1.0:
+            raise ValueError(f"p must lie in [0, 1], got {p}")
+        w = None
+        if weights is not None:
+            w = torch.as_tensor(weights)
+            if w.shape != (m,) or not (w.dtype.is_floating_point or w.dtype in (torch.int32, torch.int64)):
+                raise ValueError(f"weights must be a real tensor [{m}], got {w.dtype} {tuple(w.shape)}")
+            w = w.to(torch.float64)
+            if not bool(torch.isfinite(w).all() & (w >= 0).all() & (w.sum() > 0)):   # one synchronisation
+                raise ValueError("weights must be finite and non-negative with a positive sum")
+        if rows.device.type != "cuda":
+            raise ValueError(f"rows must be on a CUDA device, got {rows.device}")
+        if not rows.is_contiguous() or rows.data_ptr() % 16:
+            raise ValueError("rows must be contiguous and 16-byte aligned")
+        cdf = None
+        if w is not None:
+            w = w.to(rows.device)
+            # the running maximum keeps the prefix sum non-decreasing and a zero-weight slot level with the one before
+            # it, whatever order the device scan adds in
+            cdf = torch.cummax(torch.where(w > 0, torch.cumsum(w, 0), torch.zeros_like(w)), 0).values.contiguous()
+        self.rows, self.cdf, self.p, self.m = rows, cdf, p, m
+        self.row_bytes = rows.shape[1]
+        self._c = _lib.ResetPoolC(rows.data_ptr(), m, cdf.data_ptr() if cdf is not None else None, p)
+
+
 class RoboRugbyVecEnv:
     def __init__(self, env_id="RoboRugbySimpleDuel-v2", num_envs=4096, preset="GAME", device="cuda:0", seed=0,
                  env_offset=0, time_limit=True, auto_reset=True, out_dtype=torch.float32, strict_reset=True,
@@ -226,17 +268,20 @@ class RoboRugbyVecEnv:
         _lib.check(self.lib.rr_assign_balls(self._h, r.ctypes.data_as(C.c_void_p), len(r), out.data_ptr(), self._stream()))
         return out
 
-    def step(self, actions, final_info=False):
+    def step(self, actions, final_info=False, reset_pool=None):
         """One env-step for all envs.  actions: uint8 [N, A] (discrete ids) or float32 [N, A].  final_info=True adds to
         info what auto-reset would otherwise hide (see step_k): "final_observation" / "final_observation_grumpy" [N, D]
-        (valid where done), "TimeLimit.truncated" and "raised" (bool [N])."""
-        out = self.step_k(actions, 1, final_info=final_info)
+        (valid where done), "TimeLimit.truncated" and "raised" (bool [N]).  reset_pool (a ResetPool, see step_k) implies
+        final_info and adds "reset_slot" (int32 [N])."""
+        out = self.step_k(actions, 1, final_info=final_info, reset_pool=reset_pool)
         obs_h, obs_g, rew, done = out[:4]
         info = {"obs_grumpy": obs_g[0], "reward_grumpy": rew[0, :, 1]}
-        if final_info:
+        if len(out) > 4:
             f = out[4]
             info.update({"final_observation": f["final_obs"][0], "final_observation_grumpy": f["final_obs_grumpy"][0],
                          "TimeLimit.truncated": f["truncated"][0], "raised": f["raised"][0]})
+            if reset_pool is not None:
+                info["reset_slot"] = f["reset_slot"][0]
         return obs_h[0], rew[0, :, 0], done[0].bool(), info
 
     def _final_out(self, k):
@@ -248,7 +293,7 @@ class RoboRugbyVecEnv:
             self._bufs[key] = dict(final_obs_h=mk(k, N, D), final_obs_g=mk(k, N, D), row_flags=mk(k, N, dt=torch.uint8))
         return self._bufs[key]
 
-    def step_k(self, actions, k, join=True, final_info=False):
+    def step_k(self, actions, k, join=True, final_info=False, reset_pool=None):
         """k fused env-steps in ONE kernel launch (one per group with a sub-batch pipeline).  actions [k, N, A]; returns
         obs_h [k,N,D], obs_g, rew [k,N,2], done [k,N] (uint8).  Envs that finish are reset inside the launch (auto_reset).
         join=False (pipeline > 1 only): do not make the current stream wait for the launches; the caller joins later and
@@ -259,19 +304,40 @@ class RoboRugbyVecEnv:
         [k, N]): gym's info['TimeLimit.truncated'] and "the reference's step() raised".  A done row with neither is a real
         end of the episode.  The three buffers persist like the others and, with join=False, follow the same rule; since
         "truncated" and "raised" are computed from row_flags on the current stream, with join=False they are None: derive
-        them from row_flags after join()."""
+        them from row_flags after join().
+        reset_pool (a ResetPool; rr_step_pool): a done row's auto-reset starts the next episode from a pool row with
+        probability reset_pool.p, drawn by the pool's weights, and otherwise places the env at random.  The env becomes
+        what load_states makes of the row, except that it keeps its own incremented episode counter.  It implies
+        final_info, and the dict adds "reset_slot" [k, N] (int32, persistent like the others): the slot each row's reset
+        loaded, or -1 (no reset, or a random one).  With join=False the pool's tensors are kept alive like the actions."""
         actions = self._check_actions(actions, k)
         A = actions.shape[2]
+        if reset_pool is not None:
+            if not isinstance(reset_pool, ResetPool):
+                raise ValueError("reset_pool must be a ResetPool")
+            if reset_pool.row_bytes != self.state_row_bytes:
+                raise ValueError(f"reset_pool rows are {reset_pool.row_bytes} bytes wide, this env's rows "
+                                 f"{self.state_row_bytes} (state_row_bytes)")
+            if reset_pool.rows.device.index != self._dev_index:
+                raise ValueError(f"reset_pool rows must be on {self.device}, got {reset_pool.rows.device}")
+            if not self.cfg.auto_reset:
+                raise ValueError("reset_pool needs an env created with auto_reset=True")
+            final_info = True
         b = self._out(k)
         has_obs = self.obs_dim > 0
         f = self._final_out(k) if final_info else None
-        _lib.check(self.lib.rr_step_info(self._h, actions.data_ptr(), A, k,
-                                         b["obs_h"].data_ptr() if has_obs else None,
-                                         b["obs_g"].data_ptr() if has_obs else None,
-                                         b["rew"].data_ptr(), b["done"].data_ptr(),
-                                         f["final_obs_h"].data_ptr() if f and has_obs else None,
-                                         f["final_obs_g"].data_ptr() if f and has_obs else None,
-                                         f["row_flags"].data_ptr() if f else None, self._stream()))
+        args = (self._h, actions.data_ptr(), A, k, b["obs_h"].data_ptr() if has_obs else None,
+                b["obs_g"].data_ptr() if has_obs else None, b["rew"].data_ptr(), b["done"].data_ptr(),
+                f["final_obs_h"].data_ptr() if f and has_obs else None,
+                f["final_obs_g"].data_ptr() if f and has_obs else None, f["row_flags"].data_ptr() if f else None)
+        if reset_pool is None:
+            _lib.check(self.lib.rr_step_info(*args, self._stream()))
+        else:
+            key = ("slot", k)
+            if key not in self._bufs:
+                self._bufs[key] = torch.empty(k, self.num_envs, dtype=torch.int32, device=self.device)
+            f = dict(f, reset_slot=self._bufs[key])
+            _lib.check(self.lib.rr_step_pool(*args, C.byref(reset_pool._c), f["reset_slot"].data_ptr(), self._stream()))
         joined = True
         if self.pipeline > 1:
             if join:
@@ -280,6 +346,8 @@ class RoboRugbyVecEnv:
                 # keep every action buffer alive until the groups have read it: the groups run on the handle's own streams,
                 # which torch's stream-ordered allocator knows nothing about
                 self._inflight.append(actions)
+                if reset_pool is not None:
+                    self._inflight.append((reset_pool.rows, reset_pool.cdf))
                 joined = False
                 if len(self._inflight) > 256:   # a caller that never joins: bound what is kept alive
                     self.join()
@@ -290,6 +358,8 @@ class RoboRugbyVecEnv:
         info = dict(final_obs=f["final_obs_h"][..., :self.obs_dim], final_obs_grumpy=f["final_obs_g"][..., :self.obs_dim],
                     row_flags=fl, truncated=(fl & _lib.ROW_TRUNCATED).bool() if joined else None,
                     raised=(fl & _lib.ROW_RAISED).bool() if joined else None)
+        if reset_pool is not None:
+            info["reset_slot"] = f["reset_slot"]
         return out + (info,)
 
     def step_host(self, actions_host, k, out=None):

@@ -1,0 +1,69 @@
+// rr_emul_pool.cu — HOST execution of rr_step_pool's launch (k_step<L, OutT, true, true>): rr_emul.cu plus two exports.
+//
+// TEST INFRASTRUCTURE ONLY, built into its own test library (tests/emul/emul_pool.py).  launch_pool_t is launch_info_t
+// of rr_emul_info.cu with step_auto_reset replaced by step_pool_auto_reset (rr_sim.cuh), which k_step's pool variant
+// calls: the same pool draw, row load and start-column write, on EmulBatch columns plus a start array [3R + 2B][M].
+#include "rr_emul.cu"
+
+// One rr_step_pool launch: launch_info_t's outputs, plus slot [K][M] (the slot each row's reset loaded, or -1).
+// rows: the pool's m rows (RowLayout units), cdf NULL or m doubles, p the pool probability.
+template <int NH, int NG, int NP, int NN, bool G = false>
+static int launch_pool_t(const Consts &k, double *sf, int32_t *si, double *start, int64_t M, const double *actions, int A,
+                         int K, double *rew, int32_t *done, int32_t *err, int32_t *naughty, double *obs_h, double *obs_g,
+                         double *stats, double *final_h, double *final_g, int32_t *flags, const ResetPool &pool,
+                         int32_t *slot) {
+  using E = typename HostEnv<NH, NG, NP, NN, G>::E;
+  const int dim = obs_dim_of<E>(k.observer);
+  for (int64_t i = 0; i < M; i++) {
+    HostEnv<NH, NG, NP, NN, G> h;
+    auto &e = h.e;
+    col_load(e, k, sf, si, M, i);
+    double st[RR_NUM_STATS] = {};
+    int last_naughty = 0;
+    for (int s = 0; s < K; s++) {
+      const int64_t row = (int64_t)s * M + i;
+      unsigned cmd = 0;
+      int n_cmd = 0;
+      bool bad_action = false;
+      if (decode_before_refusal(e, k)) bad_action = !decode_actions<E::R>(k, actions + row * A, A, cmd, n_cmd);
+      StepOut o;
+      { FrameSync fs_; sim_step(e, k, cmd, n_cmd, o, !bad_action, fs_); }
+      done[row] = step_accounting(e, k, o, bad_action, st, last_naughty);
+      unsigned oerr = 0;
+      if (flags) flags[row] = (int32_t)step_row_flags(e, k, o);
+      if (done[row] && final_h) observe(e, k, 1, final_h + row * dim, oerr);
+      if (done[row] && final_g) observe(e, k, -1, final_g + row * dim, oerr);
+      naughty[row] = last_naughty;  // the row's own count (a pool reset then takes the loaded row's)
+      slot[row] = step_pool_auto_reset(e, k, done[row], (uint64_t)(k.env_offset + i), pool, start + i, M, last_naughty);
+      rew[2 * row] = o.rew_h; rew[2 * row + 1] = o.rew_g;
+      err[row] = (int32_t)o.step_err;
+      if (obs_h) observe(e, k, 1, obs_h + row * dim, oerr);
+      if (obs_g) observe(e, k, -1, obs_g + row * dim, oerr);
+    }
+    st[RR_STAT_REPLAYS] = e.mm(kMReplays);
+    store_columns(e, k, sf, si, M, i, last_naughty);
+    for (int q = 0; q < RR_NUM_STATS; q++) stats[i * RR_NUM_STATS + q] = st[q];
+  }
+  return 0;
+}
+
+extern "C" {
+
+void emul_launch_pool(const rr_config *cfg, double *sf, int32_t *si, double *start, int64_t M, const double *actions,
+                      int n_actions, int K, double *rew, int32_t *done, int32_t *err, int32_t *naughty, double *obs_h,
+                      double *obs_g, double *stats, double *final_h, double *final_g, int32_t *flags, const uint64_t *rows,
+                      int64_t m, const double *cdf, double p, int32_t *slot) {
+  Consts k = make_consts(*cfg);
+  k.n_actions = n_actions;
+  const ResetPool pool{rows, cdf, m, p};
+  EMUL_DISPATCH(cfg, launch_pool_t, k, sf, si, start, M, actions, n_actions, K, rew, done, err, naughty, obs_h, obs_g,
+                stats, final_h, final_g, flags, pool, slot);
+}
+
+// pool_draw for n (global env index, episode) pairs: slot[j], or -1 for a random reset
+void emul_pool_draw(uint64_t seed, const uint64_t *env, const uint32_t *episode, int64_t n, int64_t m, const double *cdf,
+                    double p, int64_t *slot) {
+  const ResetPool pool{nullptr, cdf, m, p};
+  for (int64_t j = 0; j < n; j++) slot[j] = pool_draw(pool, seed, env[j], episode[j]);
+}
+}
