@@ -27,7 +27,15 @@ def main():
     agent = VecDQNAgent(env.obs_dim, n_actions=8, batch_size=a.batch, device="cuda:0")
     train(env, agent, 20, a.learn_every)  # warm-up (cuBLAS handles, allocator)
     env.clear_stats()
-    out = train(env, agent, a.steps, a.learn_every, log_every=50)
+    out = train(env, agent, a.steps, a.learn_every, log_every=50, episode_returns=True)
+    # the reference's per-episode line (Training_DQN_pytorch.py:364-371), for the last episode that ended
+    rets, avg = out.pop("episode_returns"), out.pop("avg_return_100")
+    out.pop("avg_return_100_grumpy")
+    out["episodes_ended"] = len(rets)
+    if len(rets):
+        out["avg_return_100"] = float(avg[-1])
+        print(f"episode {len(rets) - 1} score {float(rets[-1, 0]):.2f} average score {float(avg[-1]):.2f}",
+              file=sys.stderr)
     out["config"] = vars(a)
     print(json.dumps(out))
 

@@ -360,6 +360,31 @@ int rr_step_pool(rr_sim *s, const void *actions_dev, int32_t n_actions, int32_t 
                  void *obs_g_dev, void *rew_dev, uint8_t *done_dev, void *final_obs_h_dev, void *final_obs_g_dev,
                  uint8_t *row_flags_dev, const rr_reset_pool *pool, int32_t *reset_slot_dev, void *stream);
 
+/* rr_step_pool plus each finished episode's result, which the auto-reset otherwise clears inside the launch: what a
+ * per-episode logger (gym's Monitor / RecordEpisodeStatistics) records, exact for episodes continued from pool rows.
+ * A row COUNTS AN EPISODE exactly when rr_get_stats adds 1 to RR_STAT_EPISODES for it: done = 1, not an
+ * RR_ERR_STEP_AFTER_DONE refusal, and the episode was not counted before (the episode-counted bit, which a reset or
+ * rr_set_state clears and a saved row carries).  Three optional device buffers, written on EVERY row:
+ *   ep_return_dev  double [K][N][2] (happy, grumpy), fp64 whatever out_f64 is: on a counting row the episode's return
+ *                  as RR_STAT_RETURN_* adds it (the fp64 step-order sum of its rewards, rows that raised adding 0, a pool
+ *                  row's saved return included); 0.0 on every other row, so the rows sum to the statistics' returns.
+ *   ep_length_dev  int32 [K][N]: on a counting row the step counter RR_STAT_LENGTH adds (a pool row's steps included);
+ *                  -1 on every other row.  0 is a length, not a marker: a bad action as the first step after a reset
+ *                  ends an episode of length 0.
+ *   ep_goals_dev   int32 [K][N][4], goal_scoring = 1 only: on a counting row what rr_goal_state reports for the state
+ *                  the row ended in, before the auto-reset: happy goal score, grumpy goal score, destroyed bits (bit 0
+ *                  happy, bit 1 grumpy), alive-ball bits; zeros on every other row.
+ * The outputs do not depend on the sub-batch pipeline, env_offset sharding or how K is split over launches.  pool may be
+ * NULL (the rr_step_info kernels); with all three pointers NULL this is rr_step_pool, and setting them changes no other
+ * output.  Rows are written as 128-bit stores when a buffer is 16-byte aligned and its per-step row is a multiple of 16
+ * bytes (ep_length: N a multiple of 4).
+ * RR_E_INVALID, nothing launched: rr_step_pool's argument errors; ep_return_dev not 8-byte aligned; ep_length_dev or
+ * ep_goals_dev not 4-byte aligned; ep_goals_dev on a handle without goal_scoring. */
+int rr_step_episodes(rr_sim *s, const void *actions_dev, int32_t n_actions, int32_t k_steps, void *obs_h_dev,
+                     void *obs_g_dev, void *rew_dev, uint8_t *done_dev, void *final_obs_h_dev, void *final_obs_g_dev,
+                     uint8_t *row_flags_dev, const rr_reset_pool *pool, int32_t *reset_slot_dev, double *ep_return_dev,
+                     int32_t *ep_length_dev, int32_t *ep_goals_dev, void *stream);
+
 /* Goal bookkeeping (goal_scoring = 1) to HOST; any pointer may be NULL.  alive[N]: bit b = ball b still in play;
  * score[N][2]: Goal.get_score() of the happy and the grumpy goal (RR_Goal.py:87-88); destroyed[N]: bit 0 happy goal,
  * bit 1 grumpy goal (Goal.is_destroyed, :90-91); dwell[N][2][B]: steps ball b has stayed inside that goal's triangle

@@ -83,6 +83,8 @@ SIGNATURES = {
     "rr_save_states": (C.c_int, [_vp, _vp, _i64, _vp, _vp]),
     "rr_load_states": (C.c_int, [_vp, _vp, _i64, _vp, _vp]),
     "rr_step_pool": (C.c_int, [_vp, _vp, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, C.POINTER(ResetPoolC), _vp, _vp]),
+    "rr_step_episodes": (C.c_int, [_vp, _vp, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp, C.POINTER(ResetPoolC), _vp,
+                                   _vp, _vp, _vp, _vp]),
     "rr_goal_state": (C.c_int, [_vp, _vp, _vp, _vp, _vp]),
     "rr_error_mask": (C.c_int, [_vp, _vp, _i32]),
     "rr_last_naughty": (C.c_int, [_vp, _vp]),

@@ -144,9 +144,16 @@ struct StepArgs {
   void *final_obs_h, *final_obs_g;  // rr_step_info: out_t [K][N][D], written on done rows only (k_step<L, OutT, true>)
   uint8_t *row_flags;               // rr_step_info: RR_ROW_* [K][N]
 };
+// rr_step_episodes (k_step<L, OutT, true> and the pool variant): each row's episode result, or NULL.  A struct of its
+// own, so that the default variants keep their parameter block.
+struct InfoStepArgs : StepArgs {
+  double *ep_return;   // [K][N][2]; vec bit 6: its rows can be written with 128-bit stores
+  int32_t *ep_length;  // [K][N]; vec bit 7
+  int32_t *ep_goals;   // [K][N][4] (goal scoring only); vec bit 8
+};
 // rr_step_pool (k_step<L, OutT, true, true>): the pool, the handle's start columns its resets write, and the slot rows.
 // A struct of its own, so that the other variants keep their parameter block.
-struct PoolStepArgs : StepArgs {
+struct PoolStepArgs : InfoStepArgs {
   double *start;        // [3R + 2B][N]
   ResetPool pool;
   int32_t *reset_slot;  // [K][N] or NULL; vec bit 5: its rows can be written with 128-bit stores
@@ -161,11 +168,13 @@ __device__ __forceinline__ double warp_sum(double v) {
 // The fused multi-step kernel: K env-steps per launch, auto-reset inside.  Padding threads of the
 // last block (i >= N) run the control flow without an env so that the per-frame barrier is uniform.
 // INFO: also report every row's RR_ROW_* flags and, on done rows, the terminal observation taken before the auto-reset
-// (rr_step_info).  A template switch, not a run-time branch: the default kernels keep their registers and stack.
+// (rr_step_info), and each row's episode result taken at the same point (rr_step_episodes).  A template switch, not a
+// run-time branch: the default kernels keep their registers and stack.
 // POOL (with INFO): a done row's auto-reset may load a row of a reset pool instead (rr_step_pool, pool_reset).
 template <class L, typename OutT, bool INFO = false, bool POOL = false>
 __global__ void __launch_bounds__(L::kMaxBlock, L::kStepBlocksPerSM) k_step(const __grid_constant__ Consts k,
-    const __grid_constant__ typename std::conditional<POOL, PoolStepArgs, StepArgs>::type a) {
+    const __grid_constant__ typename std::conditional<POOL, PoolStepArgs,
+                                                      typename std::conditional<INFO, InfoStepArgs, StepArgs>::type>::type a) {
   static_assert(INFO || !POOL, "the pool variant reports rr_step_info's outputs as well");
   using E = typename L::E;
   constexpr int R = E::R;
@@ -239,6 +248,30 @@ __global__ void __launch_bounds__(L::kMaxBlock, L::kStepBlocksPerSM) k_step(cons
           if (!dst) continue;
           if (live && done_flag) observe(e, k, team, ob, oerr);
           warp_store_rows<OutT>(dst + (row - lane) * dim, ob, dim, live && done_flag, false, nullptr, lane);
+        }
+      }
+      // the episode's result on the row that counted it, before the auto-reset clears it: written on every row, so
+      // staged like the results below
+      if (a.ep_return || a.ep_length || a.ep_goals) {
+        const int lane = threadIdx.x & 31;
+        const bool full = __all_sync(0xffffffffu, live);
+        const int64_t row0 = row - lane;
+        void *stage = (char *)(rr_smem + L::kTrigDoubles + E::kDoubles * (size_t)blockDim.x) + L::kStageBytes * (threadIdx.x >> 5);
+        const bool counted = live && o.counted;
+        if (a.ep_return) {
+          const double er[2] = {counted ? e.ret_h : 0.0, counted ? e.ret_g : 0.0};
+          warp_store_rows<double>(a.ep_return + row0 * 2, er, 2, live, full && (a.vec & 64u), stage, lane);
+        }
+        if (a.ep_length) {
+          const int32_t el[1] = {counted ? (int32_t)e.step : -1};
+          warp_store_rows<int32_t>(a.ep_length + row0, el, 1, live, full && (a.vec & 128u), stage, lane);
+        }
+        if constexpr (E::kGoals) {
+          if (a.ep_goals) {
+            int32_t eg[4] = {0, 0, 0, 0};
+            if (counted) goal_report(e.alive(), e.scored(), E::B, eg);
+            warp_store_rows<int32_t>(a.ep_goals + row0 * 4, eg, 4, live, full && (a.vec & 256u), stage, lane);
+          }
         }
       }
     }
@@ -1221,10 +1254,11 @@ int rr_step(rr_sim *s, const void *actions, int32_t n_actions, int32_t k_steps, 
   return rr_step_info(s, actions, n_actions, k_steps, obs_h, obs_g, rew, done, nullptr, nullptr, nullptr, stream);
 }
 
-// rr_step_info, and rr_step_pool when `pool` is given (its checks made by the caller)
+// rr_step_info, and rr_step_episodes when `pool` or an episode output is given (their checks made by the caller)
 static int step_launch(rr_sim *s, const void *actions, int32_t n_actions, int32_t k_steps, void *obs_h, void *obs_g,
                        void *rew, uint8_t *done, void *final_obs_h, void *final_obs_g, uint8_t *row_flags,
-                       const rr_reset_pool *pool, int32_t *reset_slot, void *stream) {
+                       const rr_reset_pool *pool, int32_t *reset_slot, double *ep_return, int32_t *ep_length,
+                       int32_t *ep_goals, void *stream) {
   if (!s) return fail(RR_E_INVALID, "null handle");
   int rc = check_actions(s, n_actions, k_steps);
   if (rc) return rc;
@@ -1236,7 +1270,7 @@ static int step_launch(rr_sim *s, const void *actions, int32_t n_actions, int32_
   if (misaligned(final_obs_h, osz) || misaligned(final_obs_g, osz))
     return fail(RR_E_INVALID, "final observation buffers must be aligned to their element type");
   const bool pooled = pool != nullptr;
-  const bool info = pooled || final_obs_h || final_obs_g || row_flags;
+  const bool info = pooled || final_obs_h || final_obs_g || row_flags || ep_return || ep_length || ep_goals;
   ON_DEVICE(s->device);
   cudaStream_t st = (cudaStream_t)stream;
   Consts k = s->k;
@@ -1251,11 +1285,18 @@ static int step_launch(rr_sim *s, const void *actions, int32_t n_actions, int32_
   if ((((uintptr_t)actions) & 3u) == 0) vec |= 8u;
   if (rows16(row_flags, (size_t)s->N)) vec |= 16u;
   if (rows16(reset_slot, (size_t)s->N * 4)) vec |= 32u;
+  if (rows16(ep_return, (size_t)s->N * 16)) vec |= 64u;
+  if (rows16(ep_length, (size_t)s->N * 4)) vec |= 128u;
+  if (rows16(ep_goals, (size_t)s->N * 16)) vec |= 256u;
   PoolStepArgs pa{};
   if (pooled) pa.pool = ResetPool{(const uint64_t *)pool->rows_dev, pool->cdf_dev, pool->m, pool->p_pool};
   pa.start = s->start;
   pa.reset_slot = reset_slot;
-  StepArgs &a = pa;  // what the other variants take
+  pa.ep_return = ep_return;
+  pa.ep_length = ep_length;
+  pa.ep_goals = ep_goals;
+  InfoStepArgs &ia = pa;  // what the INFO variants take
+  StepArgs &a = pa;       // what the default variants take
   a = StepArgs{s->sf, s->si, s->stats, actions, obs_h, obs_g, rew, done, s->N, k_steps, vec, 0, final_obs_h, final_obs_g, row_flags};
   const bool game = s->cfg.preset == RR_PRESET_GAME, goals = s->cfg.goal_scoring != 0, f64 = s->cfg.out_f64 != 0;
   // one stream-ordered launch per call over more envs than 384-thread blocks cover in one wave: 448-thread blocks
@@ -1270,8 +1311,8 @@ static int step_launch(rr_sim *s, const void *actions, int32_t n_actions, int32_
       const size_t sm = LTYPE::smem_bytes(blk);                                                              \
       if (pooled && f64) k_step<LTYPE, double, true, true><<<(unsigned)nblocks, blk, sm, on>>>(k, pa);       \
       else if (pooled) k_step<LTYPE, float, true, true><<<(unsigned)nblocks, blk, sm, on>>>(k, pa);          \
-      else if (info && f64) k_step<LTYPE, double, true><<<(unsigned)nblocks, blk, sm, on>>>(k, a);           \
-      else if (info) k_step<LTYPE, float, true><<<(unsigned)nblocks, blk, sm, on>>>(k, a);                   \
+      else if (info && f64) k_step<LTYPE, double, true><<<(unsigned)nblocks, blk, sm, on>>>(k, ia);          \
+      else if (info) k_step<LTYPE, float, true><<<(unsigned)nblocks, blk, sm, on>>>(k, ia);                  \
       else if (f64) k_step<LTYPE, double><<<(unsigned)nblocks, blk, sm, on>>>(k, a);                         \
       else k_step<LTYPE, float><<<(unsigned)nblocks, blk, sm, on>>>(k, a);                                   \
     } while (0)
@@ -1311,12 +1352,20 @@ static int step_launch(rr_sim *s, const void *actions, int32_t n_actions, int32_
 int rr_step_info(rr_sim *s, const void *actions, int32_t n_actions, int32_t k_steps, void *obs_h, void *obs_g, void *rew,
                  uint8_t *done, void *final_obs_h, void *final_obs_g, uint8_t *row_flags, void *stream) {
   return step_launch(s, actions, n_actions, k_steps, obs_h, obs_g, rew, done, final_obs_h, final_obs_g, row_flags, nullptr,
-                     nullptr, stream);
+                     nullptr, nullptr, nullptr, nullptr, stream);
 }
 
 int rr_step_pool(rr_sim *s, const void *actions, int32_t n_actions, int32_t k_steps, void *obs_h, void *obs_g, void *rew,
                  uint8_t *done, void *final_obs_h, void *final_obs_g, uint8_t *row_flags, const rr_reset_pool *pool,
                  int32_t *reset_slot, void *stream) {
+  return rr_step_episodes(s, actions, n_actions, k_steps, obs_h, obs_g, rew, done, final_obs_h, final_obs_g, row_flags, pool,
+                          reset_slot, nullptr, nullptr, nullptr, stream);
+}
+
+int rr_step_episodes(rr_sim *s, const void *actions, int32_t n_actions, int32_t k_steps, void *obs_h, void *obs_g,
+                     void *rew, uint8_t *done, void *final_obs_h, void *final_obs_g, uint8_t *row_flags,
+                     const rr_reset_pool *pool, int32_t *reset_slot, double *ep_return, int32_t *ep_length,
+                     int32_t *ep_goals, void *stream) {
   if (!s) return fail(RR_E_INVALID, "null handle");
   if (pool) {
     if (!pool->rows_dev) return fail(RR_E_INVALID, "reset pool: rows_dev is null");
@@ -1327,8 +1376,12 @@ int rr_step_pool(rr_sim *s, const void *actions, int32_t n_actions, int32_t k_st
     if (!s->cfg.auto_reset) return fail(RR_E_INVALID, "reset pool: the handle was created with auto_reset = 0");
   }
   if (misaligned(reset_slot, 4)) return fail(RR_E_INVALID, "reset_slot must be 4-byte aligned");
+  if (misaligned(ep_return, 8)) return fail(RR_E_INVALID, "ep_return must be 8-byte aligned");
+  if (misaligned(ep_length, 4) || misaligned(ep_goals, 4))
+    return fail(RR_E_INVALID, "ep_length and ep_goals must be 4-byte aligned");
+  if (ep_goals && !s->cfg.goal_scoring) return fail(RR_E_INVALID, "ep_goals: the handle was created without goal_scoring");
   const int rc = step_launch(s, actions, n_actions, k_steps, obs_h, obs_g, rew, done, final_obs_h, final_obs_g, row_flags,
-                             pool, reset_slot, stream);
+                             pool, reset_slot, ep_return, ep_length, ep_goals, stream);
   if (rc || pool || !reset_slot) return rc;
   // without a pool these are rr_step_info's kernels, and no row is reset from a pool
   ON_DEVICE(s->device);
@@ -1520,17 +1573,12 @@ int rr_goal_state(rr_sim *s, int32_t *alive_host, int32_t *score_host, int32_t *
   const int B = s->cols.B;
   std::vector<int32_t> g((size_t)s->cols.G * N);
   CK(cudaMemcpy(g.data(), s->si + (size_t)s->cols.goal(0) * N, sizeof(int32_t) * g.size(), cudaMemcpyDeviceToHost));
-  const uint32_t bm = (1u << B) - 1u;
   for (int64_t i = 0; i < N; i++) {
-    const uint32_t alive = (uint32_t)g[(size_t)0 * N + i], sc = (uint32_t)g[(size_t)1 * N + i];
-    if (alive_host) alive_host[i] = (int32_t)alive;
-    int destroyed = 0;
-    for (int q = 0; q < 2; q++) {  // Goal.get_score :87-88, is_destroyed :90-91
-      const int pos = __builtin_popcount((sc >> (2 * q * B)) & bm), neg = __builtin_popcount((sc >> ((2 * q + 1) * B)) & bm);
-      if (score_host) score_host[i * 2 + q] = 500 * (pos - neg);
-      if (neg >= 3) destroyed |= 1 << q;
-    }
-    if (destroyed_host) destroyed_host[i] = destroyed;
+    int32_t r[4];
+    goal_report((uint32_t)g[(size_t)0 * N + i], (uint32_t)g[(size_t)1 * N + i], B, r);
+    if (alive_host) alive_host[i] = r[3];
+    if (score_host) { score_host[i * 2] = r[0]; score_host[i * 2 + 1] = r[1]; }
+    if (destroyed_host) destroyed_host[i] = r[2];
     if (dwell_host)
       for (int q = 0; q < 2 * B; q++) dwell_host[i * 2 * B + q] = g[(size_t)(2 + q) * N + i];
   }

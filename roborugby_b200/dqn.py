@@ -113,7 +113,15 @@ class VecDQNAgent:
         return loss.detach()
 
 
-def train(env, agent, n_steps, learn_every=1, log_every=0, drive_grumpy=False):
+def _running_mean(x, n=100):
+    """np.mean(scores[-100:]) after each episode (Training_DQN_pytorch.py:364-371), for every prefix of x."""
+    c = torch.cat((torch.zeros(1, dtype=x.dtype), x.cumsum(0)))
+    i = torch.arange(1, x.numel() + 1)
+    lo = (i - n).clamp(min=0)
+    return (c[i] - c[lo]) / (i - lo)
+
+
+def train(env, agent, n_steps, learn_every=1, log_every=0, drive_grumpy=False, episode_returns=False):
     """The reference's main loop (Training_DQN_pytorch.py:317-377) for N envs in lockstep.
 
     Per iteration, exactly as the reference does per env: an eps-greedy action for the happy observation (:333-336)
@@ -126,6 +134,12 @@ def train(env, agent, n_steps, learn_every=1, log_every=0, drive_grumpy=False):
     the first grumpy robot (robot index num_robots_happy; robots between the two get uniformly random actions, since
     a GameEnv_Simple command list cannot skip a robot, RR_EnvBase.py:617-626).
 
+    episode_returns=True also records every episode that ends (env.step(..., episode_info=True): the whole return, as
+    get_stats counts it), as the reference's loop records each episode's score (:364-371): the result adds
+    "episode_returns" (float64 [n_episodes, 2], happy and grumpy, in the order the episodes ended, envs in index order
+    within a step) and "avg_return_100" / "avg_return_100_grumpy" (float64 [n_episodes]: the mean of the last 100
+    episodes after each one, the reference's avg_score).  The rows stay on the device and are gathered every 256 steps.
+
     Returns a dict with env-steps/s measured with CUDA events around the whole loop."""
     N = env.num_envs
     has_grumpy = env.preset.num_robots_grumpy > 0
@@ -134,6 +148,12 @@ def train(env, agent, n_steps, learn_every=1, log_every=0, drive_grumpy=False):
     obs_g = env.observe()[1].clone() if has_grumpy else None   # get_game_state(int_team=TEAM_GRUMPY), :322
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     losses = []
+    ends, rets, ended = [], [], []   # per-step episode rows on the device, gathered into `ended` every 256 steps
+
+    def gather():
+        if ends:
+            ended.append(torch.stack(rets)[torch.stack(ends)])
+            ends.clear(); rets.clear()
     ev0.record()
     for it in range(n_steps):
         act = agent.choose_actions(obs)
@@ -144,7 +164,14 @@ def train(env, agent, n_steps, learn_every=1, log_every=0, drive_grumpy=False):
             cmd[:, g0] = act_g
         else:
             cmd = act.view(-1, 1)
-        obs_, rew, done, info = env.step(cmd)
+        if episode_returns:
+            obs_, rew, done, info = env.step(cmd, episode_info=True)
+            ends.append(info["_episode"])
+            rets.append(torch.stack((info["episode"]["r"], info["episode"]["r_grumpy"]), 1))
+            if len(ends) == 256:
+                gather()
+        else:
+            obs_, rew, done, info = env.step(cmd)
         agent.store(obs, act, rew, obs_, done)
         if has_grumpy:
             agent.store(obs_g, act_g, info["reward_grumpy"], info["obs_grumpy"], done)
@@ -158,6 +185,11 @@ def train(env, agent, n_steps, learn_every=1, log_every=0, drive_grumpy=False):
     ev1.record()
     torch.cuda.synchronize()
     secs = ev0.elapsed_time(ev1) * 1e-3
-    return {"env_steps": n_steps * N, "seconds": secs, "env_steps_per_s": n_steps * N / secs,
-            "transitions": n_steps * N * (2 if has_grumpy else 1),
-            "losses": losses, "epsilon": agent.epsilon, "stats": env.get_stats()}
+    out = {"env_steps": n_steps * N, "seconds": secs, "env_steps_per_s": n_steps * N / secs,
+           "transitions": n_steps * N * (2 if has_grumpy else 1),
+           "losses": losses, "epsilon": agent.epsilon, "stats": env.get_stats()}
+    if episode_returns:
+        gather()
+        r = torch.cat(ended).cpu() if ended else torch.zeros(0, 2, dtype=torch.float64)
+        out.update(episode_returns=r, avg_return_100=_running_mean(r[:, 0]), avg_return_100_grumpy=_running_mean(r[:, 1]))
+    return out

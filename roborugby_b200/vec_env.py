@@ -268,12 +268,15 @@ class RoboRugbyVecEnv:
         _lib.check(self.lib.rr_assign_balls(self._h, r.ctypes.data_as(C.c_void_p), len(r), out.data_ptr(), self._stream()))
         return out
 
-    def step(self, actions, final_info=False, reset_pool=None):
+    def step(self, actions, final_info=False, reset_pool=None, episode_info=False):
         """One env-step for all envs.  actions: uint8 [N, A] (discrete ids) or float32 [N, A].  final_info=True adds to
         info what auto-reset would otherwise hide (see step_k): "final_observation" / "final_observation_grumpy" [N, D]
         (valid where done), "TimeLimit.truncated" and "raised" (bool [N]).  reset_pool (a ResetPool, see step_k) implies
-        final_info and adds "reset_slot" (int32 [N])."""
-        out = self.step_k(actions, 1, final_info=final_info, reset_pool=reset_pool)
+        final_info and adds "reset_slot" (int32 [N]).  episode_info=True (see step_k) implies final_info and adds the
+        results of the episodes this step ended in the vector layout of gym's RecordEpisodeStatistics:
+        info["episode"] = {"r": happy return [N] (float64), "r_grumpy": [N], "l": length [N] (int32)}, valid where
+        info["_episode"] (bool [N]) is True; with goal scoring also info["episode_goals"] (int32 [N, 4])."""
+        out = self.step_k(actions, 1, final_info=final_info, reset_pool=reset_pool, episode_info=episode_info)
         obs_h, obs_g, rew, done = out[:4]
         info = {"obs_grumpy": obs_g[0], "reward_grumpy": rew[0, :, 1]}
         if len(out) > 4:
@@ -282,6 +285,12 @@ class RoboRugbyVecEnv:
                          "TimeLimit.truncated": f["truncated"][0], "raised": f["raised"][0]})
             if reset_pool is not None:
                 info["reset_slot"] = f["reset_slot"][0]
+            if episode_info:
+                er = f["episode_return"][0]
+                info["episode"] = {"r": er[:, 0], "r_grumpy": er[:, 1], "l": f["episode_length"][0]}
+                info["_episode"] = f["episode_end"][0]
+                if "episode_goals" in f:
+                    info["episode_goals"] = f["episode_goals"][0]
         return obs_h[0], rew[0, :, 0], done[0].bool(), info
 
     def _final_out(self, k):
@@ -293,7 +302,19 @@ class RoboRugbyVecEnv:
             self._bufs[key] = dict(final_obs_h=mk(k, N, D), final_obs_g=mk(k, N, D), row_flags=mk(k, N, dt=torch.uint8))
         return self._bufs[key]
 
-    def step_k(self, actions, k, join=True, final_info=False, reset_pool=None):
+    def _episode_out(self, k):
+        """Persistent rr_step_episodes buffers for k fused steps."""
+        key = ("episodes", k)
+        if key not in self._bufs:
+            N = self.num_envs
+            b = dict(episode_return=torch.empty(k, N, 2, dtype=torch.float64, device=self.device),
+                     episode_length=torch.empty(k, N, dtype=torch.int32, device=self.device))
+            if self.cfg.goal_scoring:
+                b["episode_goals"] = torch.empty(k, N, 4, dtype=torch.int32, device=self.device)
+            self._bufs[key] = b
+        return self._bufs[key]
+
+    def step_k(self, actions, k, join=True, final_info=False, reset_pool=None, episode_info=False):
         """k fused env-steps in ONE kernel launch (one per group with a sub-batch pipeline).  actions [k, N, A]; returns
         obs_h [k,N,D], obs_g, rew [k,N,2], done [k,N] (uint8).  Envs that finish are reset inside the launch (auto_reset).
         join=False (pipeline > 1 only): do not make the current stream wait for the launches; the caller joins later and
@@ -309,7 +330,14 @@ class RoboRugbyVecEnv:
         probability reset_pool.p, drawn by the pool's weights, and otherwise places the env at random.  The env becomes
         what load_states makes of the row, except that it keeps its own incremented episode counter.  It implies
         final_info, and the dict adds "reset_slot" [k, N] (int32, persistent like the others): the slot each row's reset
-        loaded, or -1 (no reset, or a random one).  With join=False the pool's tensors are kept alive like the actions."""
+        loaded, or -1 (no reset, or a random one).  With join=False the pool's tensors are kept alive like the actions.
+        episode_info=True (rr_step_episodes) implies final_info and adds each row's episode result, persistent like the
+        others: "episode_return" [k, N, 2] (float64, happy and grumpy) and "episode_length" [k, N] (int32), set on the
+        row that ended (and counted, as get_stats counts) an episode and 0.0 / -1 on every other row; the return is
+        the episode's whole return, a pool row's saved return included, and the length its step counter.  "episode_end"
+        (bool [k, N], episode_length >= 0; None with join=False, like "truncated"); with goal scoring "episode_goals"
+        [k, N, 4] (int32): the ending state's goal_state() (happy score, grumpy score, destroyed bits, alive-ball bits),
+        zeros on other rows.  It combines with reset_pool."""
         actions = self._check_actions(actions, k)
         A = actions.shape[2]
         if reset_pool is not None:
@@ -323,6 +351,8 @@ class RoboRugbyVecEnv:
             if not self.cfg.auto_reset:
                 raise ValueError("reset_pool needs an env created with auto_reset=True")
             final_info = True
+        if episode_info:
+            final_info = True
         b = self._out(k)
         has_obs = self.obs_dim > 0
         f = self._final_out(k) if final_info else None
@@ -330,14 +360,22 @@ class RoboRugbyVecEnv:
                 b["obs_g"].data_ptr() if has_obs else None, b["rew"].data_ptr(), b["done"].data_ptr(),
                 f["final_obs_h"].data_ptr() if f and has_obs else None,
                 f["final_obs_g"].data_ptr() if f and has_obs else None, f["row_flags"].data_ptr() if f else None)
-        if reset_pool is None:
+        if reset_pool is None and not episode_info:
             _lib.check(self.lib.rr_step_info(*args, self._stream()))
         else:
-            key = ("slot", k)
-            if key not in self._bufs:
-                self._bufs[key] = torch.empty(k, self.num_envs, dtype=torch.int32, device=self.device)
-            f = dict(f, reset_slot=self._bufs[key])
-            _lib.check(self.lib.rr_step_pool(*args, C.byref(reset_pool._c), f["reset_slot"].data_ptr(), self._stream()))
+            pool = slot = None
+            if reset_pool is not None:
+                key = ("slot", k)
+                if key not in self._bufs:
+                    self._bufs[key] = torch.empty(k, self.num_envs, dtype=torch.int32, device=self.device)
+                f = dict(f, reset_slot=self._bufs[key])
+                pool, slot = C.byref(reset_pool._c), f["reset_slot"].data_ptr()
+            ep = (None, None, None)
+            if episode_info:
+                f = dict(f, **self._episode_out(k))
+                ep = (f["episode_return"].data_ptr(), f["episode_length"].data_ptr(),
+                      f["episode_goals"].data_ptr() if "episode_goals" in f else None)
+            _lib.check(self.lib.rr_step_episodes(*args, pool, slot, *ep, self._stream()))
         joined = True
         if self.pipeline > 1:
             if join:
@@ -360,6 +398,11 @@ class RoboRugbyVecEnv:
                     raised=(fl & _lib.ROW_RAISED).bool() if joined else None)
         if reset_pool is not None:
             info["reset_slot"] = f["reset_slot"]
+        if episode_info:
+            info.update(episode_return=f["episode_return"], episode_length=f["episode_length"],
+                        episode_end=f["episode_length"] >= 0 if joined else None)
+            if "episode_goals" in f:
+                info["episode_goals"] = f["episode_goals"]
         return out + (info,)
 
     def step_host(self, actions_host, k, out=None):
